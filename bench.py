@@ -4,13 +4,18 @@
   degradation (blur, downsample, noise, re-upsample, normalise) + the always-on T1 target warp --
   batch 8 x 160^3 per step on each GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  `value` = samples/s with all inputs resident in HBM (host-side random
 draws and table planning INCLUDED, overlapped with the GPU through the asynchronous stream); `e2e` = the same
 through the public API with host label/image buffers copied in and the generated volumes copied out every
 step; `roofline` = the dominant kernel (warp+gamma+bias) against the measured HBM peak; `cpu_baseline` = the
 oracle port of the reference's PyTorch-CPU generator on this box's host cores.
+
+`--dump-outputs DIR` writes what the device-resident arm's last timed step handed its caller (rank 0): every tensor of
+the batch's samples and targets, stacked over the batch, as DIR/<name>.npy in float32 (see `dump_outputs`).  The
+inputs and the random streams depend on the arguments only, so two builds run with the same arguments can be
+compared output for output.
 """
 import argparse
 import json
@@ -329,6 +334,40 @@ def build_dataset(subs, device, planner="auto"):
     return ds
 
 
+DUMP_BYTES = 64_000_000
+
+
+def batch_outputs(items):
+    """The tensors a caller receives from one batch, stacked over its items: those of the samples (`input`,
+    `bias_field_log`, ...) and those of the targets (`target_T1`, ...)."""
+    out = {}
+    for _, _, _, target, sample in items:
+        for smp in sample if isinstance(sample, list) else [sample]:
+            for k, v in smp.items():
+                if torch.is_tensor(v):
+                    out.setdefault(k, []).append(v)
+        for k, v in target.items():
+            if torch.is_tensor(v):
+                out.setdefault("target_" + k, []).append(v)
+    return {k: torch.stack(v) for k, v in out.items()}
+
+
+def dump_outputs(arrays, path):
+    """Writes every array as <path>/<name>.npy in float32, DUMP_BYTES in all.  An array larger than its equal share is
+    flattened and sampled: the same seeded, sorted set of flat indices for every array of that size, so that the
+    samples of, say, `input` and `bias_field_log` are the same voxels."""
+    os.makedirs(path, exist_ok=True)
+    share = (DUMP_BYTES // max(1, len(arrays)) - 1024) // 4          # float32 values per array (1 KB for the header)
+    picks = {}
+    for name, t in sorted(arrays.items()):
+        a = t.detach().to(torch.float32).cpu().numpy()
+        if a.size > share:
+            if a.size not in picks:
+                picks[a.size] = np.sort(np.random.default_rng(0).choice(a.size, share, replace=False))
+            a = a.reshape(-1)[picks[a.size]]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -340,7 +379,13 @@ def main():
     ap.add_argument("--planner", default="auto", choices=["auto", "python", "native"])
     ap.add_argument("--lanes", type=int, default=2, help="batches in flight in the device-resident arm")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[2..4] records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step of the device-resident arm as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the CUDA path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -452,6 +497,8 @@ def main():
     barrier()
     t1 = time.perf_counter()
     gcq.__exit__()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(batch_outputs(tickets[-1].items), args.dump_outputs)
     host_s = t1 - t0
     if trace is not None and rank == 0:
         print("per-step host ms: %s" % trace, file=sys.stderr, flush=True)

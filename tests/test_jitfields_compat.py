@@ -1,11 +1,13 @@
 """brainfm_b200.interpol.jitfields_compat: the `jitfields`-shaped front end that lets the REFERENCE's own
 utils.interpol forward to libbfm (utils/interpol/backend.py:1, jitfields.py:28-95).
 
-CPU part (build container only -- needs /root/reference): the reference package is imported with our module
-installed as `jitfields` and `backend.jitfields = True`; our kernels cannot run without a GPU, so the six entry
-points of brainfm_b200.interpol.api are replaced by recorders that check the layout they receive and answer with the
+CPU part: the reference package (a checkout of the original project named by BFM_REFERENCE_ROOT, the variable
+oracle/ref_shim.py reads; skipped without one) is imported with our module installed as `jitfields` and
+`backend.jitfields = True`; our kernels cannot run without a GPU, so the six entry points of brainfm_b200.interpol.api are replaced by recorders that check the layout they receive and answer with the
 reference's native implementation.  A call that goes reference API -> reference shim -> our front end -> (recorder)
 -> back must then equal the reference's direct answer: that pins the argument marshalling in both directions.
+Without a checkout, test_front_end_marshalling pins the front end's side of it: jitfields' keyword names and
+channels-last layout in, this package's API calls and channels-first layout out, for every entry point.
 GPU part: the front end against brainfm_b200.interpol.api itself (channels-last vs channels-first)."""
 import importlib
 import os
@@ -16,13 +18,13 @@ import numpy as np
 import pytest
 import torch
 
-REF = "/root/reference/utils/interpol"
+REF = os.path.join(os.environ.get("BFM_REFERENCE_ROOT", ""), "utils", "interpol")
 
 
 @pytest.fixture(scope="module")
 def ref_interpol():
-    if not os.path.isdir(REF):
-        pytest.skip("reference checkout not present (GPU box)")
+    if not os.environ.get("BFM_REFERENCE_ROOT") or not os.path.isdir(REF):
+        pytest.skip("no checkout of the original project (set BFM_REFERENCE_ROOT)")
     import brainfm_b200.interpol.jitfields_compat as jf
     tmp = tempfile.mkdtemp(prefix="ref_interpol_")
     os.symlink(REF, os.path.join(tmp, "interpol"))          # SURVEY appendix B-6: not via utils/ (shadows logging)
@@ -116,6 +118,79 @@ def test_unbatched_and_channel_free_inputs(ref_interpol, monkeypatch):
         ref.backend.jitfields = False
     assert calls[0][1] == [(1, 6, 5, 4), (3, 3, 3, 3)]
     assert torch.equal(got, want)
+
+
+def test_front_end_marshalling(monkeypatch):
+    """Every entry point of the front end, without a GPU: the API functions are replaced by recorders that check the
+    channel-first data they receive and answer with a known channel-first tensor, which must come back in jitfields'
+    layout (channels last; pull / grad / push) or unchanged (count, spline_coeff*, resize, restrict)."""
+    import brainfm_b200.interpol.jitfields_compat as jf
+    from brainfm_b200.interpol import api
+    torch.manual_seed(0)
+    B, C, shp, oshp = 2, 3, (7, 6, 5), (4, 5, 6)
+    xl = torch.rand(B, *shp, C)
+    x = torch.movedim(xl, -1, 1)
+    grid = torch.rand(B, *oshp, 3)
+    gin = torch.rand(B, *shp, 3)
+    calls = {}
+
+    def answer(*shape):
+        return torch.arange(float(np.prod(shape))).reshape(shape)
+
+    def stub(name, out_shape, want_input, want_grid=None):
+        def run(*a, **k):
+            calls[name] = (a, k)
+            if want_input is not None:
+                assert torch.equal(a[0], want_input), name
+            if want_grid is not None:
+                assert a[1] is want_grid, name
+            return answer(*out_shape)
+        monkeypatch.setattr(api, name, run)
+
+    stub("grid_pull", (B, C, *oshp), x, grid)
+    stub("grid_grad", (B, C, *oshp, 3), x, grid)
+    stub("grid_push", (B, C, *oshp), x, gin)
+    stub("grid_count", (B, *oshp), None, None)
+    stub("spline_coeff", (B, C, *shp), x)
+    stub("spline_coeff_nd", (B, C, *shp), x)
+    stub("resize", (B, C, 9, 8, 7), x)
+    stub("restrict", (B, C, 3, 3, 2), x)
+    kw = dict(bound="dft", extrapolate=False)
+    full = dict(bound="dft", extrapolate=False, prefilter=True)
+
+    got = jf.pull(xl, grid, order=3, prefilter=True, **kw)
+    assert torch.equal(got, torch.movedim(answer(B, C, *oshp), 1, -1))
+    assert calls["grid_pull"][1] == dict(interpolation=3, **full)
+    out = torch.empty(B, *oshp, C)
+    assert jf.pull(xl, grid, order=3, out=out, **kw) is out and torch.equal(out, got)
+
+    got = jf.grad(xl, grid, order=1, prefilter=True, **kw)
+    assert torch.equal(got, torch.movedim(answer(B, C, *oshp, 3), 1, -2))
+    assert calls["grid_grad"][1] == dict(interpolation=1, **full)
+
+    got = jf.push(xl, gin, oshp, order=2, prefilter=True, **kw)
+    assert torch.equal(got, torch.movedim(answer(B, C, *oshp), 1, -1))
+    assert calls["grid_push"][0][2] == oshp and calls["grid_push"][1] == dict(interpolation=2, **full)
+
+    got = jf.count(gin, oshp, order=0, **kw)
+    assert torch.equal(got, answer(B, *oshp))
+    assert calls["grid_count"][0] == (gin, oshp) and calls["grid_count"][1] == dict(interpolation=0, **kw)
+
+    for fn, inplace in ((jf.spline_coeff, False), (jf.spline_coeff_, True)):
+        assert torch.equal(fn(x, 3, bound="dst2", dim=2), answer(B, C, *shp))
+        assert calls["spline_coeff"][1] == dict(interpolation=3, bound="dst2", dim=2, inplace=inplace)
+    for fn, inplace in ((jf.spline_coeff_nd, False), (jf.spline_coeff_nd_, True)):
+        assert torch.equal(fn(x, 5, bound="dct1", ndim=3), answer(B, C, *shp))
+        assert calls["spline_coeff_nd"][1] == dict(interpolation=5, bound="dct1", dim=3, inplace=inplace)
+
+    assert torch.equal(jf.resize(x, shape=[9, 8, 7], ndim=3, anchor="c", order=1, bound="zero", prefilter=False),
+                       answer(B, C, 9, 8, 7))
+    assert calls["resize"][1] == dict(factor=None, shape=[9, 8, 7], anchor="c", interpolation=1, prefilter=False,
+                                      bound="zero")
+    assert torch.equal(jf.restrict(x, factor=2, ndim=3, anchor="e", order=2, bound="dct2", reduce_sum=True),
+                       answer(B, C, 3, 3, 2))
+    assert calls["restrict"][1] == dict(factor=2, shape=None, anchor="e", interpolation=2, reduce_sum=True,
+                                        bound="dct2")
 
 
 @pytest.mark.gpu

@@ -1,6 +1,6 @@
 """brainfm_b200.io readers (nib.load replacement, Generator/utils.py:296-305): NIfTI-1 and MGH / MGZ files written here
-byte by byte from the formats' specifications, the reference's shipped files/gca.mgz when the reference tree is
-present, and the committed benchmark label map derived from it."""
+byte by byte from the formats' specifications, the reference's shipped files/gca.mgz when a checkout of the original
+project is named by BFM_REFERENCE_ROOT, and the committed benchmark label map derived from it."""
 import gzip
 import os
 import struct
@@ -11,7 +11,7 @@ import pytest
 from brainfm_b200 import io as bio
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-GCA = "/root/reference/files/gca.mgz"
+GCA = os.path.join(os.environ.get("BFM_REFERENCE_ROOT", ""), "files", "gca.mgz")
 
 
 def _nifti_bytes(data, endian="<", slope=0.0, inter=0.0, sform=None, pixdim=(1.0, 1.0, 1.0)):
@@ -104,7 +104,8 @@ def test_benchmark_label_map_fixture():
     assert 0.5 < (L > 0).mean() < 0.6 and L.max() == 233
 
 
-@pytest.mark.skipif(not os.path.exists(GCA), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not os.environ.get("BFM_REFERENCE_ROOT") or not os.path.exists(GCA),
+                    reason="no checkout of the original project (set BFM_REFERENCE_ROOT)")
 def test_reference_atlas_and_the_fixture_derived_from_it():
     """files/gca.mgz, the only real volume the reference ships (SURVEY.md 2.1 row 20): 256^3, integer valued 0..233,
     non-zero bounding box 152 x 176 x 184; the committed fixture is the documented crop of it."""
