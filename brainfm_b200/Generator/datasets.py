@@ -482,7 +482,7 @@ class BaseGen(Dataset):
         res_all = torch.empty((n_res, 1, *size), dtype=torch.float32, device=dev) if n_res else None
         aux_all = torch.empty((n_aux, 1, *size), dtype=torch.float32, device=dev) if n_aux else None
         # persistent scratch: syn is zero-initialised once and afterwards only ever holds finite values
-        src_pad = max(int(np.prod(j['plan'].src)) + j['plan'].src[1] * j['plan'].src[2] + j['plan'].src[2] + 9
+        src_pad = max(int(np.prod(j['plan'].src)) + j['plan'].src[1] * j['plan'].src[2] + j['plan'].src[2] + 1
                       for j in jobs)
         src_pad = 2 * ((src_pad + 3) // 4 * 4)         # room for float2 {synthetic, T1} pairs (syn_pair_ok)
         syn_ws = self._workspace('syn', B * src_pad, zero=True)
@@ -492,7 +492,7 @@ class BaseGen(Dataset):
             self._ws['syn_stride'] = src_pad
         i_bf_ws = self._workspace('i_bf', B * N)
         tmp_ws = self._workspace('tmp', B * 2 * N)
-        low_ws = self._workspace('lowres', B * N + 16)     # + slack: bulk copies end on a 16-byte boundary
+        low_ws = self._workspace('lowres', B * N)
         raw_ws = self._workspace('aux_raw', n_aux * N) if n_aux else None
         p_syn, p_ibf, p_tmp, p_low = syn_ws.data_ptr(), i_bf_ws.data_ptr(), tmp_ws.data_ptr(), low_ws.data_ptr()
         keep = [out, bfl_all, res_all, aux_all]
@@ -1005,8 +1005,8 @@ class BaseGen(Dataset):
 
     def generate_batch_fast(self, indices):
         """generate_batch through `NativePlanner.run_fast` (one library call per batch, lazily built result tuples), or
-        None when the configuration / batch needs the general path.  BFM_FAST_SUBMIT=0 disables it."""
-        if os.environ.get("BFM_FAST_SUBMIT", "1") == "0" or self.planner == 'python':
+        None when the configuration / batch needs the general path."""
+        if self.planner == 'python':
             return None
         self.cache.begin_batch()
         from .native import NativePlanner

@@ -196,7 +196,7 @@ class NativePlanner:
                 it.aux_src[c] = vol.data_ptr()
                 keys.append((mods[k_], 'f32'))
             n_aux_total += len(aux)
-            src_pad = max(src_pad, src[0] * src[1] * src[2] + src[1] * src[2] + src[2] + 9)
+            src_pad = max(src_pad, src[0] * src[1] * src[2] + src[1] * src[2] + src[2] + 1)
             metas.append((idx, dataset_name, t1_path, age, dict(mods), aux, src))
         ent = dict(items=items, metas=metas, n_aux_total=n_aux_total, src_pad=src_pad, keys=keys,
                    version=cache.version, ok=None)
@@ -320,7 +320,7 @@ class NativePlanner:
         bufs.syn_stride = src_pad
         bufs.i_bf = ds._workspace('i_bf', total * N).data_ptr()
         bufs.tmp = ds._workspace('tmp', total * 2 * N).data_ptr()
-        bufs.lowres = ds._workspace('lowres', total * N + 16).data_ptr()
+        bufs.lowres = ds._workspace('lowres', total * N).data_ptr()
         if n_aux_total:
             bufs.aux_out = aux_all.data_ptr()
             bufs.aux_raw = ds._workspace('aux_raw', n_aux_total * N).data_ptr()
@@ -387,7 +387,7 @@ class NativePlanner:
             ds._ws['syn_stride'] = src_pad
         p_ibf = ds._workspace('i_bf', total * N).data_ptr()
         p_tmp = ds._workspace('tmp', total * 2 * N).data_ptr()
-        p_low = ds._workspace('lowres', total * N + 16).data_ptr()     # + slack: bulk copies end on a 16-byte boundary
+        p_low = ds._workspace('lowres', total * N).data_ptr()
         p_raw = ds._workspace('aux_raw', n_aux_total * N).data_ptr() if n_aux_total else 0
         outs = (_lib.PlanOut * total)()
         o_np = np.frombuffer(outs, dtype=np.uint64).reshape(total, 9)

@@ -17,8 +17,6 @@
 // a warp owns several rows so per-k table entries are loaded once, element indices are 32-bit.
 #include "common.cuh"
 
-#include <cstdlib>
-
 namespace bfm {
 
 constexpr float kBoxDelta = 1e-3f;   // bound on |computed - exact| source coordinate (see DESIGN.md)
@@ -1056,331 +1054,6 @@ k_gen_warp_pk(const bfm_gen_sample *__restrict__ S, const __grid_constant__ PkPa
     else warp_rows_pk<0>(sh, t1F, t1B, rpb, P.s[blockIdx.z], P.one);
 }
 
-
-// ---------------------------------------------------------------------------------------------- warp, tile mode (TMA)
-// k_gen_warp_pk is bound by L1 data-pipe wavefronts (profiles/r2_ncu_full_v1_summary.csv: 81 % of peak): the 16 lanes
-// of a 64-bit gather request run along z in the SOURCE volume and cross ~2.5 cache lines, and every line is one
-// wavefront.  Here a CTA owns a compact 8 x 8 x 16 tile of the OUTPUT grid, whose source footprint is a small brick
-// (12 x 12 x 18 voxels on average for the reference's parameter ranges).  Per tile:
-//   A. every thread evaluates the coordinates of its 4 voxels (2 row pairs, same f32x2 arithmetic as the pair kernel)
-//      and the block reduces the integer bounding box of the taps;
-//   B. one warp copies the brick's rows (x, y, z0 .. z0 + ez) of the float2 {synthetic, target} volume into shared
-//      memory with bulk asynchronous copies (cp.async.bulk global -> shared, completion on an mbarrier): no register
-//      staging, no L1 wavefronts;
-//   C. the 8 taps of a voxel are 64-bit SHARED loads: the 16 lanes of a half warp read consecutive z of one brick row,
-//      whose pitch is a multiple of 8 voxels (16 banks), so a request is ~1 wavefront per half warp instead of ~2.5.
-// Tiles whose brick does not fit the shared-memory budget gather straight from global memory (same arithmetic).
-// The zoom passes of the small random grids are evaluated once per CTA for its 8 planes x 8 rows and reused by the
-// s2 / 16 tiles along z.
-constexpr int kTI = 8, kTJ = 8, kTK = 16;
-
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long *bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(unsigned long long *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long *bar, uint32_t parity) {
-    uint32_t done;
-    do {
-        asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-                     : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    } while (!done);
-}
-// bulk asynchronous copy global -> shared (TMA engine, 1-D): bytes and both addresses are multiples of 16
-__device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, uint32_t bytes, unsigned long long *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst_smem)), "l"(__cvta_generic_to_global(src_gmem)), "r"(bytes), "r"(smem_u32(bar))
-                 : "memory");
-}
-
-struct TileShared {
-    bfm_gen_sample sd;
-    alignas(8) unsigned long long mbar;
-    int bb[2][6];                   // tap bounding box of the current / next tile: min x, y, z, max x, y, z (crop relative)
-    float red[8][2];
-};
-
-template <int FIELD>
-__device__ __forceinline__ void warp_tile(TileShared &sh, float *dyn, const int NF, const int NB, const int brick_bytes,
-                                          const PkSample &c, const float one) {
-    const bfm_gen_sample &s = sh.sd;
-    const bfm_deform &d = s.d;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int s0 = d.size[0], s1 = d.size[1], s2 = d.size[2];
-    const int i0 = (s.x_count > 0 ? s.x_begin : 0) + blockIdx.y * kTI, j0 = blockIdx.x * kTJ;
-    const int i_end = (s.x_count > 0 ? s.x_begin + s.x_count : s0);
-    const float *__restrict__ bfsmall = s.bfsmall;
-    const int nf = FIELD == 1 ? d.fs[2] : 0, fw = nf * 3;
-    const int nb = bfsmall ? s.bs[2] : 0;
-    // dynamic shared memory: f2 [8][4][NF][8] | b2 [8][4][NB][2] | brick (aliased by the first-pass rows t1F / t1B)
-    float *f2 = dyn;
-    float *b2 = f2 + kTI * (kTJ / 2) * NF * 8;
-    float *brick = b2 + kTI * (kTJ / 2) * NB * 2;
-    const bool photo = d.photo != 0;
-    {   // ---- zoom passes 1 (axis 0) and 2 (axis 1) for the 8 planes x 8 rows of this CTA        utils.py:239-243
-        const int nF1 = FIELD == 1 ? d.fs[1] * fw : 0, nB1 = nb ? s.bs[1] * nb : 0;
-        float *t1F = brick, *t1B = brick + kTI * nF1;
-        for (int il = warp; il < kTI; il += (blockDim.x >> 5)) {
-            const int i = min(i0 + il, s0 - 1);
-            if (FIELD == 1) {
-                const int lo = __ldg(d.ftab.lo[0] + i), hi = __ldg(d.ftab.hi[0] + i);
-                const float wl = __ldg(d.ftab.wl[0] + i), wh = __ldg(d.ftab.wh[0] + i);
-                const float *a = d.fsmall + lo * nF1, *b = d.fsmall + hi * nF1;
-                for (int q = lane; q < nF1; q += 32) t1F[il * nF1 + q] = lerp_rn(wl, __ldg(a + q), wh, __ldg(b + q));
-            }
-            if (nb) {
-                const int lo = __ldg(s.btab.lo[0] + i), hi = __ldg(s.btab.hi[0] + i);
-                const float wl = __ldg(s.btab.wl[0] + i), wh = __ldg(s.btab.wh[0] + i);
-                const float *a = bfsmall + lo * nB1, *b = bfsmall + hi * nB1;
-                for (int q = lane; q < nB1; q += 32) t1B[il * nB1 + q] = lerp_rn(wl, __ldg(a + q), wh, __ldg(b + q));
-            }
-        }
-        __syncthreads();
-        for (int row = warp; row < kTI * kTJ; row += (blockDim.x >> 5)) {
-            const int il = row / kTJ, jl = row - il * kTJ;
-            const int j = min(j0 + jl, s1 - 1);
-            if (FIELD == 1) {
-                const int lo = __ldg(d.ftab.lo[1] + j) * fw, hi = __ldg(d.ftab.hi[1] + j) * fw;
-                const float wl = __ldg(d.ftab.wl[1] + j), wh = __ldg(d.ftab.wh[1] + j);
-                const float *src = t1F + il * nF1;
-                float *dst = f2 + ((il * (kTJ / 2) + (jl >> 1)) * NF) * 8 + (jl & 1);
-                for (int q = lane; q < fw + 3; q += 32) {                 // node nf duplicates node nf - 1
-                    const int node = q / 3, ch = q - node * 3, e = min(node, nf - 1) * 3 + ch;
-                    const float v = lerp_rn(wl, src[lo + e], wh, src[hi + e]);
-                    dst[node * 8 + ch * 2] = (photo && ch == 1) ? 0.f : v;       // datasets.py:211-212
-                }
-            }
-            if (nb) {
-                const int lo = __ldg(s.btab.lo[1] + j) * nb, hi = __ldg(s.btab.hi[1] + j) * nb;
-                const float wl = __ldg(s.btab.wl[1] + j), wh = __ldg(s.btab.wh[1] + j);
-                const float *src = t1B + il * nB1;
-                float *dst = b2 + ((il * (kTJ / 2) + (jl >> 1)) * NB) * 2 + (jl & 1);
-                for (int q = lane; q <= nb; q += 32) {
-                    const int e = min(q, nb - 1);
-                    dst[q * 2] = lerp_rn(wl, src[lo + e], wh, src[hi + e]);
-                }
-            }
-        }
-        if (tid == 0) {
-            mbar_init(&sh.mbar, 1);
-            for (int q = 0; q < 2; ++q) {
-                sh.bb[q][0] = sh.bb[q][1] = sh.bb[q][2] = 0x7fffffff;
-                sh.bb[q][3] = sh.bb[q][4] = sh.bb[q][5] = -1;
-            }
-        }
-        __syncthreads();                       // t1F / t1B are dead from here on: the brick may overwrite them
-    }
-    const BoxRegs box = load_box(s.bbox, d.src[1], d.src[2]);
-    const int origin = box.b0 * box.n1n2 + box.b1 * box.n2 + box.b2;
-    const float2 *__restrict__ syn2 = (const float2 *)s.syn;
-    const float gamma = c.gamma;
-    float *__restrict__ i_bf = s.i_bf;
-    float *__restrict__ bfl = nb ? s.bflog_out : nullptr;
-    float *__restrict__ araw = s.aux_raw[0];
-    float amin = INFINITY, amax = -INFINITY;
-    const float mx = (float)(d.src[0] - 1), my = (float)(d.src[1] - 1), mz = (float)(d.src[2] - 1);
-    const u64 ONE = pk2(one, one);
-    const u64 NL0 = pk2(-box.l0, -box.l0), NL1 = pk2(-box.l1, -box.l1), NL2 = pk2(-box.l2, -box.l2);
-    // this thread: plane il = warp, rows 2 * pp and 2 * pp + 1 for the pairs pp = half, half + 2; column kl of the tile
-    const int il = warp, half = lane >> 4, kl = lane & 15;
-    const int i = i0 + il;
-    const bool iv = i < i_end;
-    const int ic = iv ? i : s0 - 1;
-    const float xc = __fsub_rn((float)ic, c.ctr[0]);
-    const u64 XC = pk2(xc, xc);
-    const int plane_in = ic * s1, plane_out = (s.flip ? s0 - 1 - ic : ic) * s1;
-    uint32_t parity = 0;
-    int cur = 0;                               // which tap box this tile reduces into
-
-    for (int k0 = 0; k0 < s2; k0 += kTK, cur ^= 1) {
-        int *bb = sh.bb[cur];
-        const int k = k0 + kl;
-        const bool kv = k < s2;
-        const int kk = kv ? k : s2 - 1;
-        int zlo = 0, blo = 0;
-        u64 ZWL = 0, ZWH = 0, BWL = 0, BWH = 0;
-        if (FIELD == 1) {
-            zlo = __ldg(d.ftab.lo[2] + kk);
-            const float wl = __ldg(d.ftab.wl[2] + kk), wh = __ldg(d.ftab.wh[2] + kk);
-            ZWL = pk2(wl, wl); ZWH = pk2(wh, wh);
-        }
-        if (nb) {
-            blo = __ldg(s.btab.lo[2] + kk);
-            const float wl = __ldg(s.btab.wl[2] + kk), wh = __ldg(s.btab.wh[2] + kk);
-            BWL = pk2(wl, wl); BWH = pk2(wh, wh);
-        }
-        const float zc = __fsub_rn((float)kk, c.ctr[2]);
-        const u64 ZC = pk2(zc, zc);
-        // ---- A. coordinates of the 4 voxels, tap box of the tile
-        int tap[4];                              // crop-relative (ix, iy, iz) packed 10 bits each; -1 = masked
-        float ax[4], ay[4], az[4], blv[4];
-        int lo0 = 0x7fffffff, lo1 = 0x7fffffff, lo2 = 0x7fffffff, hi0 = -1, hi1 = -1, hi2 = -1;
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-            const int pp = half + 2 * q, j = j0 + 2 * pp;
-            u64 X1 = XC, Y1 = pk2(__fsub_rn((float)j, c.ctr[1]), __fsub_rn((float)(j + 1), c.ctr[1])), Z1 = ZC;
-            if (FIELD == 1) {                                    // third pass (axis 2), utils.py:244-246
-                const float4 *fn = (const float4 *)(f2 + ((il * (kTJ / 2) + pp) * NF + zlo) * 8);
-                const float4 l01 = fn[0], h01 = fn[2];
-                const float2 l2 = *(const float2 *)(fn + 1), h2 = *(const float2 *)(fn + 3);
-                const u64 F0 = fma2(mul2(ZWH, pk2(h01.x, h01.y)), ONE, mul2(ZWL, pk2(l01.x, l01.y)));
-                const u64 F1 = fma2(mul2(ZWH, pk2(h01.z, h01.w)), ONE, mul2(ZWL, pk2(l01.z, l01.w)));
-                const u64 F2 = fma2(mul2(ZWH, f2u(h2)), ONE, mul2(ZWL, f2u(l2)));
-                X1 = add2(X1, F0); Y1 = add2(Y1, F1); Z1 = add2(Z1, F2);
-            }
-            auto affine = [&](const float a0, const float a1, const float a2, const float cc) {
-                const u64 m0 = mul2(pk2(a0, a0), X1), m1 = mul2(pk2(a1, a1), Y1), m2 = mul2(pk2(a2, a2), Z1);
-                return add2(fma2(m2, ONE, fma2(m1, ONE, m0)), pk2(cc, cc));
-            };
-            const float2 px = upk2(affine(c.A[0], c.A[1], c.A[2], c.c2[0]));
-            const float2 py = upk2(affine(c.A[3], c.A[4], c.A[5], c.c2[1]));
-            const float2 pz = upk2(affine(c.A[6], c.A[7], c.A[8], c.c2[2]));
-            auto clampf = [](float v, float hi) { v = v < 0.f ? 0.f : v; return v > hi ? hi : v; };
-            const float2 rx = upk2(add2(pk2(clampf(px.x, mx), clampf(px.y, mx)), NL0));
-            const float2 ry = upk2(add2(pk2(clampf(py.x, my), clampf(py.y, my)), NL1));
-            const float2 rz = upk2(add2(pk2(clampf(pz.x, mz), clampf(pz.y, mz)), NL2));
-            const float rxa[2] = {rx.x, rx.y}, rya[2] = {ry.x, ry.y}, rza[2] = {rz.x, rz.y};
-            float2 bl = make_float2(0.f, 0.f);
-            if (nb) {
-                const float2 *bn = (const float2 *)(b2 + ((il * (kTJ / 2) + pp) * NB + blo) * 2);
-                bl = upk2(fma2(mul2(BWH, f2u(bn[1])), ONE, mul2(BWL, f2u(bn[0]))));
-            }
-            blv[2 * q] = bl.x; blv[2 * q + 1] = bl.y;
-#pragma unroll
-            for (int r = 0; r < 2; ++r) {
-                const int v = 2 * q + r;
-                const bool ok = (rxa[r] > 0.f) & (rya[r] > 0.f) & (rza[r] > 0.f) & (rxa[r] <= box.h0) &
-                                (rya[r] <= box.h1) & (rza[r] <= box.h2) & (j + r < s1) & iv & kv;
-                const int ix = __float2int_rd(rxa[r]), iy = __float2int_rd(rya[r]), iz = __float2int_rd(rza[r]);
-                ax[v] = __fsub_rn(rxa[r], (float)ix); ay[v] = __fsub_rn(rya[r], (float)iy);
-                az[v] = __fsub_rn(rza[r], (float)iz);
-                tap[v] = ok ? (ix << 20) | (iy << 10) | iz : -1;
-                if (ok) {
-                    lo0 = min(lo0, ix); hi0 = max(hi0, ix); lo1 = min(lo1, iy); hi1 = max(hi1, iy);
-                    lo2 = min(lo2, iz); hi2 = max(hi2, iz);
-                }
-            }
-        }
-        lo0 = __reduce_min_sync(0xffffffffu, lo0); lo1 = __reduce_min_sync(0xffffffffu, lo1);
-        lo2 = __reduce_min_sync(0xffffffffu, lo2); hi0 = __reduce_max_sync(0xffffffffu, hi0);
-        hi1 = __reduce_max_sync(0xffffffffu, hi1); hi2 = __reduce_max_sync(0xffffffffu, hi2);
-        if (lane == 0 && hi0 >= 0) {
-            atomicMin(&bb[0], lo0); atomicMin(&bb[1], lo1); atomicMin(&bb[2], lo2);
-            atomicMax(&bb[3], hi0); atomicMax(&bb[4], hi1); atomicMax(&bb[5], hi2);
-        }
-        __syncthreads();
-        // ---- B. brick geometry (uniform) and the bulk copies
-        const bool any = bb[3] >= 0;
-        // rows start on an even ABSOLUTE z (16-byte aligned source address): z0 may be -1 relative to the crop
-        const int x0 = bb[0], y0 = bb[1], z0 = any ? ((box.b2 + bb[2]) & ~1) - box.b2 : 0;
-        const int ex = bb[3] + 2 - x0, ey = bb[4] + 2 - y0;
-        const int ez = (bb[5] + 2 - z0 + 1) & ~1;             // voxels per row actually copied (16-byte granules)
-        if (tid == 0) {                                       // the other box: everybody is done reading it
-            int *nb_ = sh.bb[cur ^ 1];
-            nb_[0] = nb_[1] = nb_[2] = 0x7fffffff;
-            nb_[3] = nb_[4] = nb_[5] = -1;
-        }
-        const int pz = (ez + 7) & ~7;                         // row pitch: 8 voxels = 16 banks
-        const int rows = ex * ey;
-        const bool fits = any && (int64_t)rows * pz * 8 <= brick_bytes;
-        if (fits) {
-            // every warp issues its share of the row copies (a bulk copy takes uniform operands: the lanes of a warp
-            // issue one after the other, so the rows are dealt round-robin to the 8 warps)
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy accesses of the brick are done
-            if (tid == 0) mbar_arrive_expect_tx(&sh.mbar, (uint32_t)(rows * ez * 8));
-            const float2 *src0 = syn2 + origin + z0;
-            const int nw = blockDim.x >> 5;
-            for (int r = lane * nw + warp; r < rows; r += 32 * nw) {
-                const int rx_ = r / ey, ry_ = r - rx_ * ey;
-                bulk_g2s(brick + (size_t)r * pz * 2, src0 + (x0 + rx_) * box.n1n2 + (y0 + ry_) * box.n2,
-                         (uint32_t)(ez * 8), &sh.mbar);
-            }
-        }
-        if (fits) {
-            mbar_wait(&sh.mbar, parity);
-            parity ^= 1;
-        }
-        // ---- C. gathers (shared bricks, or global memory when the brick did not fit), interpolation, epilogue
-        const int sy = pz, sx = ey * pz;                       // brick strides in float2
-#pragma unroll
-        for (int v = 0; v < 4; ++v) {
-            const int pp = half + 2 * (v >> 1), j = j0 + 2 * pp + (v & 1);
-            const bool ok = tap[v] >= 0;
-            const int ix = (tap[v] >> 20) & 1023, iy = (tap[v] >> 10) & 1023, iz = tap[v] & 1023;
-            u64 t[8];                               // {synthetic, target} at 000 001 100 101 010 011 110 111
-            if (fits) {
-                const float2 *b00 = (const float2 *)brick + (ok ? ((ix - x0) * ey + (iy - y0)) * pz + (iz - z0) : 0);
-                t[0] = f2u(b00[0]); t[1] = f2u(b00[1]);
-                t[2] = f2u(b00[sx]); t[3] = f2u(b00[sx + 1]);
-                t[4] = f2u(b00[sy]); t[5] = f2u(b00[sy + 1]);
-                t[6] = f2u(b00[sx + sy]); t[7] = f2u(b00[sx + sy + 1]);
-            } else {
-                const float2 *b00 = syn2 + (ok ? origin + ix * box.n1n2 + iy * box.n2 + iz : origin);
-                const float2 *b10 = b00 + box.n1n2, *b01 = b00 + box.n2, *b11 = b10 + box.n2;
-                t[0] = f2u(__ldg(b00)); t[1] = f2u(__ldg(b00 + 1));
-                t[2] = f2u(__ldg(b10)); t[3] = f2u(__ldg(b10 + 1));
-                t[4] = f2u(__ldg(b01)); t[5] = f2u(__ldg(b01 + 1));
-                t[6] = f2u(__ldg(b11)); t[7] = f2u(__ldg(b11 + 1));
-            }
-            const u64 AX = pk2(ax[v], ax[v]), AY = pk2(ay[v], ay[v]), AZ = pk2(az[v], az[v]);
-            const u64 c00 = fma2(AX, sub2(t[2], t[0]), t[0]), c01 = fma2(AX, sub2(t[3], t[1]), t[1]);
-            const u64 c10 = fma2(AX, sub2(t[6], t[4]), t[4]), c11 = fma2(AX, sub2(t[7], t[5]), t[5]);
-            const u64 c0 = fma2(AY, sub2(c10, c00), c00), c1 = fma2(AY, sub2(c11, c01), c01);
-            const float2 vv = upk2(fma2(AZ, sub2(c1, c0), c0));
-            float val = ok ? vv.x : 0.f;
-            const float a = ok ? vv.y : 0.f;
-            val = fmaxf(val, 0.f);                                    // datasets.py:411
-            val = 300.f * fast_pow(val * (1.f / 300.f), gamma);       // utils.py:568-572
-            if (nb) val *= ex2_approx(blv[v] * 1.4426950408889634f);
-            if (kv && iv && j < s1) {
-                const int pr = (plane_in + j) * s2 + k;
-                i_bf[pr] = val;
-                if (bfl) bfl[(plane_out + j) * s2 + k] = blv[v];
-                araw[pr] = a;                                         // read_and_deform_image: raw warp + min/max
-                amin = fminf(amin, a);
-                amax = fmaxf(amax, a);
-            }
-        }
-        __syncthreads();                                   // the brick is free again
-    }
-    {
-        const float lo = warp_min(amin), hi = warp_max(amax);
-        if (lane == 0) { sh.red[warp][0] = lo; sh.red[warp][1] = hi; }
-        __syncthreads();
-        if (tid < 2) {
-            float v = sh.red[0][tid];
-            for (int w = 1; w < (int)(blockDim.x >> 5); ++w)
-                v = (tid & 1) ? fmaxf(v, sh.red[w][tid]) : fminf(v, sh.red[w][tid]);
-            if (tid & 1) atomicMax(s.aux_mm + tid, f2ord(v));
-            else atomicMin(s.aux_mm + tid, f2ord(v));
-        }
-    }
-}
-
-#ifndef WARP_TILE_MINB
-#define WARP_TILE_MINB 2
-#endif
-__global__ void __launch_bounds__(256, WARP_TILE_MINB)
-k_gen_warp_tile(const bfm_gen_sample *__restrict__ S, const __grid_constant__ PkParams P, int NF, int NB,
-                int brick_bytes) {
-    extern __shared__ __align__(128) float dyn[];
-    __shared__ TileShared sh;
-    const int b = P.base + blockIdx.z;
-    {
-        const bfm_gen_sample *sp = S + b;
-        if (!use_pairs(*sp)) return;
-        const int nx = sp->x_count > 0 ? sp->x_count : sp->d.size[0];
-        if ((int)blockIdx.y * kTI >= nx || (int)blockIdx.x * kTJ >= sp->d.size[1]) return;
-    }
-    stage_desc(&sh.sd, S + b);
-    if (sh.sd.d.fsmall) warp_tile<1>(sh, dyn, NF, NB, brick_bytes, P.s[blockIdx.z], P.one);
-    else warp_tile<0>(sh, dyn, NF, NB, brick_bytes, P.s[blockIdx.z], P.one);
-}
-
-
 // Undegraded resolution class (resolution == thickness == the training resolution: identity band, new_size == size):
 // the banded pass is a copy and the zoom back is the identity (weights exactly 1 and 0), so those samples take
 // k_gen_identity -- noise + clamp straight from i_bf into `out` -- instead of the band and upsample kernels.
@@ -1391,9 +1064,6 @@ __host__ __device__ __forceinline__ bool is_identity_sample(const bfm_gen_sample
 }
 
 // ---------------------------------------------------------------------------------------------- resample
-#ifndef BAND_UNROLL
-#define BAND_UNROLL 4
-#endif
 // One banded pass.  Axis 0/1: a thread owns VEC consecutive z outputs (128-bit loads when VEC == 4); the tap
 // weight is uniform across the warp.  Axis 2: a thread owns one output, taps are contiguous.
 #ifndef BAND_UNROLL
@@ -1647,7 +1317,6 @@ __global__ void __launch_bounds__(256) k_gen_identity(const bfm_gen_sample *__re
 #define UPS_MINB 8
 #endif
 constexpr int kUR = UPS_ROWS;     // output rows per block
-constexpr int kFinishGroup = 0;   // samples per upsample -> normalise group (0 = whole batch); see bfm_gen_finish
 
 // myzoom_torch(lowres, 1/factors): three sequential 2-tap passes (axis 0, 1, 2), each `wl*a + wh*b` separately rounded.
 // Block = (x plane i, kUR output rows), thread = k.  The first pass (axis 0) of the low-res rows under the block's
@@ -1711,105 +1380,6 @@ __global__ void __launch_bounds__(160, UPS_MINB) k_gen_upsample(const bfm_gen_sa
             o[(size_t)r * s2] = v;
             hi = fmaxf(hi, v);
         }
-    }
-    hi = warp_max(hi);
-    if (lane == 0) red[warp] = hi;
-    __syncthreads();
-    if (tid == 0) {
-        for (int w = 1; w < nwarps; ++w) hi = fmaxf(hi, red[w]);
-        atomicMax((int *)s.maxval, __float_as_int(hi));               // values >= 0: bit order == float order
-    }
-}
-
-// Persistent form of k_gen_upsample with the low-res rows prefetched by the bulk-copy engine (opt-in, BFM_UPSAMPLE_BULK=1:
-// parity-green but slower than the plain kernel on B200, see bfm_gen_finish).  A block walks items
-// (x plane i, kUB output rows); while it computes item n from shared memory, one elected thread has already queued the
-// two contiguous row blocks of item n + 1 (low-res planes lo(i) and hi(i), rows y0 .. y1) as cp.async.bulk copies that
-// complete on an mbarrier -- the loads that left k_gen_upsample long-scoreboard bound (profiles/
-// r2_ncu_upsample_v2_summary.csv: 4.7 stalled warps per issue) are off the critical path and cost no registers.
-// Bulk copies need 16-byte aligned addresses and sizes: a row block starts at an arbitrary float of the low-res volume,
-// so the copy starts at the aligned float below it (offset kept per item) and ends at the aligned float above its end;
-// `lowres` must therefore be followed by >= 3 readable floats (bfm.h).  Arithmetic and results: identical to
-// k_gen_upsample.
-constexpr int kUB = 16;           // output rows per item
-struct UpsItem { int oa, ob, y0, ny, i, j0; float wl, wh; };
-
-__global__ void __launch_bounds__(160, 3) k_gen_upsample_bulk(const bfm_gen_sample *__restrict__ S, int cap) {
-    extern __shared__ __align__(16) float smem[];
-    __shared__ alignas(8) unsigned long long full[2];
-    __shared__ UpsItem item[2];
-    __shared__ float red[8];
-    __shared__ int ylo_s[kUB], yhi_s[kUB];
-    __shared__ float ywl_s[kUB], ywh_s[kUB];
-    const bfm_gen_sample &s = S[blockIdx.y];
-    if (is_identity_sample(s)) return;                  // k_gen_identity (resample stage) already wrote `out`
-    const int s0 = s.d.size[0], s1 = s.d.size[1], s2 = s.d.size[2];
-    const int ly = s.new_size[1], lz = s.new_size[2];
-    const int n_rg = (s1 + kUB - 1) / kUB, n_items = s0 * n_rg;
-    if ((int)blockIdx.x >= n_items) return;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nwarps = blockDim.x >> 5;
-    float *raw = smem, *t1 = smem + 4 * cap;            // raw[stage][plane lo / hi][cap], t1[cap]
-    const bfm_zoom_tab &u = s.utab;
-    const float *__restrict__ lowres = s.lowres;
-    if (tid == 0) { mbar_init(&full[0], 1); mbar_init(&full[1], 1); }
-    __syncthreads();
-    auto issue = [&](int t, int st) {                   // one thread: describe item t and queue its two copies
-        UpsItem it;
-        it.i = t / n_rg;
-        it.j0 = (t - it.i * n_rg) * kUB;
-        const int j1 = min(it.j0 + kUB, s1);
-        it.y0 = __ldg(u.lo[1] + it.j0);
-        it.ny = __ldg(u.hi[1] + j1 - 1) - it.y0 + 1;
-        const int lo = __ldg(u.lo[0] + it.i), hi = __ldg(u.hi[0] + it.i);
-        it.wl = __ldg(u.wl[0] + it.i); it.wh = __ldg(u.wh[0] + it.i);
-        const int64_t a = ((int64_t)lo * ly + it.y0) * lz, b = ((int64_t)hi * ly + it.y0) * lz;
-        it.oa = (int)(a & 3); it.ob = (int)(b & 3);
-        const int n = it.ny * lz;
-        const uint32_t ba = (uint32_t)((it.oa + n + 3) & ~3) * 4u, bb = (uint32_t)((it.ob + n + 3) & ~3) * 4u;
-        item[st] = it;
-        mbar_arrive_expect_tx(&full[st], ba + bb);
-        bulk_g2s(raw + (st * 2 + 0) * cap, lowres + (a - it.oa), ba, &full[st]);
-        bulk_g2s(raw + (st * 2 + 1) * cap, lowres + (b - it.ob), bb, &full[st]);
-    };
-    if (tid == 0) issue(blockIdx.x, 0);
-    __syncthreads();
-    float *__restrict__ outp = s.out;
-    const int flip = s.flip;
-    float hi = 0.f;
-    int n = 0;
-    for (int t = blockIdx.x; t < n_items; t += gridDim.x, ++n) {
-        const int st = n & 1;
-        if (tid == 0 && t + (int)gridDim.x < n_items) issue(t + gridDim.x, st ^ 1);   // raw[st ^ 1] was consumed before barrier A of item n - 1
-        const UpsItem it = item[st];
-        const int rows = min(kUB, s1 - it.j0);
-        if (tid < rows) {
-            const int j = it.j0 + tid;
-            ylo_s[tid] = (__ldg(u.lo[1] + j) - it.y0) * lz; yhi_s[tid] = (__ldg(u.hi[1] + j) - it.y0) * lz;
-            ywl_s[tid] = __ldg(u.wl[1] + j); ywh_s[tid] = __ldg(u.wh[1] + j);
-        }
-        mbar_wait(&full[st], (uint32_t)((n >> 1) & 1));
-        {   // first zoom pass (axis 0): shared -> shared
-            const float *ra = raw + (st * 2 + 0) * cap + it.oa, *rb = raw + (st * 2 + 1) * cap + it.ob;
-            const int cnt = it.ny * lz;
-            for (int q = tid; q < cnt; q += blockDim.x) t1[q] = lerp_rn(it.wl, ra[q], it.wh, rb[q]);
-        }
-        __syncthreads();                                                         // barrier A
-        const int plane_out = (flip ? s0 - 1 - it.i : it.i) * s1;
-        for (int k = tid; k < s2; k += blockDim.x) {
-            const int zlo = __ldg(u.lo[2] + k), zhi = __ldg(u.hi[2] + k);
-            const float zwl = __ldg(u.wl[2] + k), zwh = __ldg(u.wh[2] + k);
-            float *__restrict__ o = outp + (size_t)(plane_out + it.j0) * s2 + k;
-#pragma unroll 4
-            for (int r = 0; r < rows; ++r) {
-                const float *a = t1 + ylo_s[r], *b = t1 + yhi_s[r];
-                const float wl = ywl_s[r], wh = ywh_s[r];
-                const float vl = lerp_rn(wl, a[zlo], wh, b[zlo]), vh = lerp_rn(wl, a[zhi], wh, b[zhi]);
-                const float v = lerp_rn(zwl, vl, zwh, vh);
-                o[(size_t)r * s2] = v;
-                hi = fmaxf(hi, v);
-            }
-        }
-        __syncthreads();                                                         // barrier B: t1 / row tables reusable
     }
     hi = warp_max(hi);
     if (lane == 0) red[warp] = hi;
@@ -1974,9 +1544,8 @@ int bfm_gen_gmm(const bfm_gen_sample *h, const bfm_gen_sample *d, int B, void *s
         // and enough blocks for ~2 waves of 148 SMs x 8 resident blocks: with one block per plane a batch of 8 x 160
         // planes is 1.08 waves (a nearly empty second wave).  Measured per sample: 1 tile 13.8 us, 2: 12.6, 4: 13.1,
         // 8: 14.4 (the 512-entry table is staged per block).
-        static const int tiles_env = getenv("BFM_GMM_TILES") ? atoi(getenv("BFM_GMM_TILES")) : 0;
         const int64_t want = (2LL * 148 * 8 + (int64_t)max_n0 * B - 1) / ((int64_t)max_n0 * B);
-        const int tiles = tiles_env > 0 ? tiles_env : (int)min((int64_t)8, max((int64_t)1, want));
+        const int tiles = (int)min((int64_t)8, max((int64_t)1, want));
         k_gen_gmm_planes<<<dim3(tiles, max_n0, B), 256, 0, (cudaStream_t)stream>>>(d);
         rc = check_launch("bfm_gen_gmm");
         if (rc) return rc;
@@ -2073,52 +1642,6 @@ int bfm_gen_warp(const bfm_gen_sample *h, const bfm_gen_sample *d, int B, void *
     BFM_LAUNCH_WARP(3, 3, false)
     BFM_LAUNCH_WARP(4, 0, true)
 #undef BFM_LAUNCH_WARP
-    // tile mode (k_gen_warp_tile): bulk-copied source bricks in shared memory.  Opt-in (BFM_WARP_TILE=1): with one
-    // cp.async.bulk per brick row the copy engine's per-request cost dominates (profiles/README.md, r2 tile runs)
-    const char *te = getenv("BFM_WARP_TILE"), *bk = getenv("BFM_BRICK_KB");      // read per call: tests toggle them
-    const int tile_env = te ? atoi(te) : 0, brick_kb = bk ? atoi(bk) : 48;
-    bool tile_ok = any_pk && tile_env != 0;
-    int NF = 1, NB = 1, t1_floats = 0;
-    if (tile_ok) {
-        for (int b = 0; b < B; ++b) {
-            const bfm_gen_sample &sm = h[b];
-            if (!use_pairs(sm)) continue;
-            if (sm.d.src[0] > 1023 || sm.d.src[1] > 1023 || sm.d.src[2] > 1023) tile_ok = false;
-            const int nf = sm.d.fsmall ? sm.d.fs[2] : 0, nbz = sm.bfsmall ? sm.bs[2] : 0;
-            NF = max(NF, nf + 1); NB = max(NB, nbz + 1);
-            t1_floats = max(t1_floats, kTI * ((sm.d.fsmall ? sm.d.fs[1] * nf * 3 : 0) + (sm.bfsmall ? sm.bs[1] * nbz : 0)));
-        }
-    }
-    const int brick_bytes = max(brick_kb * 1024, (t1_floats * 4 + 127) / 128 * 128);
-    const size_t tile_smem = (size_t)(kTI * (kTJ / 2) * (NF * 8 + NB * 2)) * 4 + brick_bytes;
-    if (tile_ok && tile_smem > 200 * 1024) tile_ok = false;
-    if (tile_ok) {
-        static size_t attr = 0;
-        if (tile_smem > attr) {
-            cudaFuncSetAttribute(k_gen_warp_tile, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem);
-            attr = tile_smem;
-        }
-        const dim3 tgrid((s1 + kTJ - 1) / kTJ, (s0 + kTI - 1) / kTI, 1);
-        for (int base = 0; base < B; base += kPkBatch) {
-            const int nbk = min(kPkBatch, B - base);
-            PkParams P;
-            bool any = false;
-            for (int q = 0; q < nbk; ++q) {
-                const bfm_gen_sample &sm = h[base + q];
-                any |= use_pairs(sm);
-                for (int a = 0; a < 9; ++a) P.s[q].A[a] = sm.d.A[a];
-                for (int a = 0; a < 3; ++a) { P.s[q].c2[a] = sm.d.c2[a]; P.s[q].ctr[a] = sm.d.ctr[a]; }
-                P.s[q].gamma = sm.gamma;
-            }
-            if (!any) continue;
-            P.one = 1.0f;
-            P.base = base;
-            k_gen_warp_tile<<<dim3(tgrid.x, tgrid.y, nbk), 256, tile_smem, st>>>(d, P, NF, NB, brick_bytes);
-            rc = check_launch("bfm_gen_warp");
-            if (rc) return rc;
-        }
-        return BFM_OK;
-    }
     if (any_pk) {
         if (smem > 40 * 1024)
             cudaFuncSetAttribute(k_gen_warp_pk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -2150,8 +1673,8 @@ int bfm_gen_resample(const bfm_gen_sample *h, const bfm_gen_sample *d, int B, vo
     int maxp = 0;
     for (int b = 0; b < B; ++b) maxp = h[b].n_band > maxp ? h[b].n_band : maxp;
     // persistent blocks: ~16 per SM over the whole batch
-    static const int bps = getenv("BFM_BAND_BLOCKS_PER_SM") ? atoi(getenv("BFM_BAND_BLOCKS_PER_SM")) : 16;
-    const int64_t band_blocks = max((int64_t)8, (int64_t)((int64_t)bps * 148 + B - 1) / B);
+    constexpr int kBandBlocksPerSM = 16;
+    const int64_t band_blocks = max((int64_t)8, (int64_t)((int64_t)kBandBlocksPerSM * 148 + B - 1) / B);
     const int zk_cap = 96 * 1024;          // shared memory of k_gen_band_z (2 blocks per SM)
     static bool attr_done = false;
     if (!attr_done) {
@@ -2232,55 +1755,23 @@ int bfm_gen_finish(const bfm_gen_sample *h, const bfm_gen_sample *d, int B, void
     }
     const size_t smem = (size_t)ny * lz * sizeof(float);
     if (smem > 200 * 1024) return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen_finish: low-res rows too long for shared memory");
-    // bulk form: 2 stages x 2 planes of raw rows + the first-pass buffer, each `cap` floats
-    int nyb = 1;
-    for (int b = 0; b < B; ++b)
-        nyb = max(nyb, min(h[b].new_size[1], (int)((int64_t)kUB * h[b].new_size[1] / h[b].d.size[1]) + 3));
-    const int cap = ((nyb * lz + 8) + 3) & ~3;
-    const size_t smem_bulk = (size_t)5 * cap * sizeof(float);
-    // opt-in: measured 21.6 instead of 18.4 us per sample for the finish stage (3 persistent blocks of 5 warps per SM,
-    // two barriers + one mbarrier wait per item, the first pass re-read from shared memory) -- the plain kernel's many
-    // small blocks hide the row loads better than the prefetch does
-    const char *be = getenv("BFM_UPSAMPLE_BULK");                 // read per call: tests toggle it
-    const int bulk_env = be ? atoi(be) : 0;
-    const bool bulk = bulk_env != 0 && smem_bulk <= 72 * 1024;
     if (s0 > 65535 || B > 65535) return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen_finish: grid too large");
     if (smem > 40 * 1024)
         cudaFuncSetAttribute(k_gen_upsample, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     cudaStream_t st = (cudaStream_t)stream;
     const int threads = min(160, (s2 + 31) / 32 * 32);
     const int64_t plane = (int64_t)s1 * s2;
-    // Groups of samples: the unnormalised volumes k_gen_upsample writes (4 B/voxel) are still in the 126 MB L2 when
-    // k_gen_normalize reads them back if a group stays well below L2 size.  BFM_FINISH_GROUP overrides (0 = whole batch).
-    static const int group_env = getenv("BFM_FINISH_GROUP") ? atoi(getenv("BFM_FINISH_GROUP")) : -1;
-    int G = group_env < 0 ? kFinishGroup : group_env;
-    if (G <= 0 || G > B) G = B;
-    for (int b0 = 0; b0 < B; b0 += G) {
-        const int n = B - b0 < G ? B - b0 : G;
-        if (bulk) {
-            static size_t attr = 0;
-            if (smem_bulk > attr) {
-                cudaFuncSetAttribute(k_gen_upsample_bulk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bulk);
-                attr = smem_bulk;
-            }
-            const int items = s0 * ((s1 + kUB - 1) / kUB);
-            const int per = min(items, max(8, (3 * 148 + n - 1) / n));          // ~3 persistent blocks per SM over the group
-            k_gen_upsample_bulk<<<dim3(per, n), threads, smem_bulk, st>>>(d + b0, cap);
-        } else {
-            k_gen_upsample<<<dim3((s1 + kUR - 1) / kUR, s0, n), threads, smem, st>>>(d + b0, lz, ny);
-        }
+    k_gen_upsample<<<dim3((s1 + kUR - 1) / kUR, s0, B), threads, smem, st>>>(d, lz, ny);
+    rc = check_launch("bfm_gen_finish");
+    if (rc) return rc;
+    if (vec) {
+        k_gen_normalize<4><<<dim3((unsigned)((plane / 4 + 255) / 256), s0, B), 256, 0, st>>>(d);
         rc = check_launch("bfm_gen_finish");
         if (rc) return rc;
-        if (vec) {
-            k_gen_normalize<4><<<dim3((unsigned)((plane / 4 + 255) / 256), s0, n), 256, 0, st>>>(d + b0);
-            rc = check_launch("bfm_gen_finish");
-            if (rc) return rc;
-        }
-        if (scalar) {
-            k_gen_normalize<1><<<dim3((unsigned)((plane + 255) / 256), s0, n), 256, 0, st>>>(d + b0);
-            rc = check_launch("bfm_gen_finish");
-            if (rc) return rc;
-        }
+    }
+    if (scalar) {
+        k_gen_normalize<1><<<dim3((unsigned)((plane + 255) / 256), s0, B), 256, 0, st>>>(d);
+        rc = check_launch("bfm_gen_finish");
     }
     return rc;
 }
@@ -2289,21 +1780,10 @@ int bfm_gen_run(const bfm_gen_sample *h, const bfm_gen_sample *d, int B, void *s
     int rc;
     if ((rc = bfm_gen_plan(h, d, B, stream))) return rc;
     if ((rc = bfm_gen_bbox(h, d, B, stream))) return rc;
-    // The volume-sized stages run over groups of samples (sample-major order) so that what one stage writes is
-    // still in the 126 MB L2 when the next one reads it (syn: 4-8 B/voxel of the crop, i_bf / raw targets / out:
-    // 4 B/voxel each).  BFM_GEN_GROUP overrides the group size (0 = the whole batch, stage-major).
-    static const int group_env = getenv("BFM_GEN_GROUP") ? atoi(getenv("BFM_GEN_GROUP")) : -1;
-    int G = group_env;
-    if (G < 0) G = B;               // default decided by measurement (profiles/): see DESIGN.md
-    if (G <= 0 || G > B) G = B;
-    for (int b0 = 0; b0 < B; b0 += G) {
-        const int n = B - b0 < G ? B - b0 : G;
-        if ((rc = bfm_gen_gmm(h + b0, d + b0, n, stream))) return rc;
-        if ((rc = bfm_gen_warp(h + b0, d + b0, n, stream))) return rc;
-        if ((rc = bfm_gen_resample(h + b0, d + b0, n, stream))) return rc;
-        if ((rc = bfm_gen_finish(h + b0, d + b0, n, stream))) return rc;
-    }
-    return BFM_OK;
+    if ((rc = bfm_gen_gmm(h, d, B, stream))) return rc;
+    if ((rc = bfm_gen_warp(h, d, B, stream))) return rc;
+    if ((rc = bfm_gen_resample(h, d, B, stream))) return rc;
+    return bfm_gen_finish(h, d, B, stream);
 }
 
 }  // extern "C"

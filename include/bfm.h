@@ -225,7 +225,7 @@ typedef struct bfm_gen_sample {
     float noise_std;
     const float *eps_noise; /* injected, low-res shaped, or NULL => Philox */
     float *tmp[2];          /* ping-pong scratch, each >= prod(size) floats */
-    float *lowres;          /* (new_size), 16-byte aligned, followed by >= 3 readable floats (bulk copies of row blocks) */
+    float *lowres;          /* (new_size), 16-byte aligned */
     int new_size[3];
     /* back to the training grid + normalise */
     bfm_zoom_tab utab;      /* tables of myzoom_torch(lowres, 1/factors), lengths size[d] */
@@ -261,10 +261,9 @@ typedef struct bfm_gen_sample {
        there is no bias field (bfsmall == NULL, Generator/utils.py:575-577). */
     int real_input;
     /* Pair mode.  syn_pair_ok != 0: `syn` has room for TWICE the floats (2 * (source volume + tail padding), zeroed
-       once by the caller; tail padding >= src[1]*src[2] + src[2] + 9 elements: bfm_gen_warp's tile mode copies whole
-       16-byte aligned row segments of the pairs into shared memory).  For samples with exactly one real-image target, no mixing, a synthetic input, src[2] % 4
-       == 0 and no full-resolution field, bfm_gen_gmm then writes {synthetic value, aux_src[0] value} PAIRS
-       (float2 per source voxel) and bfm_gen_warp gathers both volumes with one 64-bit load per trilinear tap
+       once by the caller; tail padding >= src[1]*src[2]+src[2]+1 pairs, as for the unpaired path).  For samples with
+       exactly one real-image target, no mixing, a synthetic input, src[2] % 4 == 0 and no full-resolution field,
+       bfm_gen_gmm then writes {synthetic value, aux_src[0] value} PAIRS (float2 per source voxel) and bfm_gen_warp gathers both volumes with one 64-bit load per trilinear tap
        (k_gen_warp_pk: half the load requests of the two-volume gather, packed f32x2 arithmetic).  Results are
        identical to the unpaired path. */
     int syn_pair_ok;

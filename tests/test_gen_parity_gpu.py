@@ -111,32 +111,11 @@ def test_svf_integration_is_bit_exact(name):
     assert [int(v) for v in grid[3:]] == orc.deform["lo"] + orc.deform["hi"]
 
 
-@pytest.mark.parametrize("name", ["g64_s0", "g64_s2", "g160_s0", "g64_s5_lowres", "g64_s3"])
-def test_bulk_prefetched_upsample_is_identical(name, monkeypatch):
-    """k_gen_upsample_bulk (persistent blocks, low-res row blocks prefetched with cp.async.bulk + mbarrier, unaligned
-    row blocks copied from the 16-byte boundary below; BFM_UPSAMPLE_BULK=1) against k_gen_upsample: bit-identical."""
-    _, orc = oracle_case(name)
-    monkeypatch.setenv("BFM_UPSAMPLE_BULK", "1")
-    got_b, _, _ = cuda_case(name, orc.log)
-    monkeypatch.setenv("BFM_UPSAMPLE_BULK", "0")
-    got_p, _, _ = cuda_case(name, orc.log)
-    a, b = mg.flatten(got_b), mg.flatten(got_p)
-    for k, v in a.items():
-        if isinstance(v, torch.Tensor):
-            assert torch.equal(v, b[k]), k
-
-
-@pytest.mark.parametrize("tile", ["1", "0", "tiny-bricks"])
 @pytest.mark.parametrize("name", ["g64_s0", "g64_s2", "g160_s0", "g64_s5_lowres"])
-def test_pair_mode_is_identical_to_the_unpaired_gather(name, tile, monkeypatch):
-    """k_gen_warp_tile (bulk-copied source bricks in shared memory; BFM_WARP_TILE=1), k_gen_warp_pk
-    (float2 {synthetic, T1} gathers from global memory, packed f32x2 arithmetic; BFM_WARP_TILE=0, the default) and the tile
-    kernel with a 4 KB brick budget (most tiles take its global-memory fallback) against k_gen_warp<1, 0>: same
+def test_pair_mode_is_identical_to_the_unpaired_gather(name, monkeypatch):
+    """k_gen_warp_pk (float2 {synthetic, T1} gathers, packed f32x2 arithmetic) against k_gen_warp<1, 0>: same
     operations, bit-identical outputs."""
     _, orc = oracle_case(name)
-    monkeypatch.setenv("BFM_WARP_TILE", "0" if tile == "0" else "1")
-    if tile == "tiny-bricks":
-        monkeypatch.setenv("BFM_BRICK_KB", "4")
     got_pk, ds, _ = cuda_case(name, orc.log)
     assert ds.pair_mode and ds._last_descs[0][0].syn_pair_ok == 1
     monkeypatch.setenv("BFM_PAIR_MODE", "0")

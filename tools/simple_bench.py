@@ -41,7 +41,7 @@ def main():
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / STEPS
     print(json.dumps({"ms_per_step": round(ms, 4), "samples_per_s": round(bench.BATCH / ms * 1e3, 1),
-                      "group": os.environ.get("BFM_GEN_GROUP"), "streams": nstreams, "lib": os.path.basename(_lib.LIB_PATH)}))
+                      "streams": nstreams, "lib": os.path.basename(_lib.LIB_PATH)}))
 
 
 if __name__ == "__main__":
