@@ -23,7 +23,7 @@ from ..draws import HostDraws
 from ..plan import Arena, band_host, device_tables, set_zoom_tab, zoom_newsize
 from . import constants as K
 from .utils import (DeformDict, DeformPlan, _stream, fast_3D_interp_torch, make_affine_matrix, myzoom_torch,
-                    read_and_deform_image, resolution_sampler)
+                    read_and_deform_image, resolution_sampler, scratch_stride)
 
 ct_brightness_group = {
     'darker': [4, 5, 14, 15, 24, 31, 72],
@@ -490,10 +490,11 @@ class BaseGen(Dataset):
             if 'syn_stride' in self._ws:
                 syn_ws.zero_()
             self._ws['syn_stride'] = src_pad
-        i_bf_ws = self._workspace('i_bf', B * N)
-        tmp_ws = self._workspace('tmp', B * 2 * N)
-        low_ws = self._workspace('lowres', B * N)
-        raw_ws = self._workspace('aux_raw', n_aux * N) if n_aux else None
+        Np = scratch_stride(N)
+        i_bf_ws = self._workspace('i_bf', B * Np)
+        tmp_ws = self._workspace('tmp', B * 2 * Np)
+        low_ws = self._workspace('lowres', B * Np)
+        raw_ws = self._workspace('aux_raw', n_aux * Np) if n_aux else None
         p_syn, p_ibf, p_tmp, p_low = syn_ws.data_ptr(), i_bf_ws.data_ptr(), tmp_ws.data_ptr(), low_ws.data_ptr()
         keep = [out, bfl_all, res_all, aux_all]
         results = []
@@ -531,7 +532,7 @@ class BaseGen(Dataset):
                 s.bfsmall = p['bfsmall_dev'] if 'bfsmall_dev' in p else arena.put(bfs)
                 s.bs[:] = bfs.shape
                 s.btab = tables.zoom_tab(bfs.shape, size)
-            s.i_bf = p_ibf + 4 * b * N
+            s.i_bf = p_ibf + 4 * b * Np
             sample = {}
             if job['want_bflog']:
                 s.bflog_out = bfl_all[k_bfl].data_ptr()
@@ -572,9 +573,9 @@ class BaseGen(Dataset):
                 e = p['eps_noise'].to(dev).contiguous()
                 keep.append(e)
                 s.eps_noise = e.data_ptr()
-            s.tmp[0] = p_tmp + 4 * (2 * b) * N
-            s.tmp[1] = p_tmp + 4 * (2 * b + 1) * N
-            s.lowres = p_low + 4 * b * N
+            s.tmp[0] = p_tmp + 4 * (2 * b) * Np
+            s.tmp[1] = p_tmp + 4 * (2 * b + 1) * Np
+            s.lowres = p_low + 4 * b * Np
             s.new_size[:] = new
             s.utab = tables.zoom_tab(new, size, inverse=True)
             s.maxval, _ = arena.reserve(16)
@@ -591,7 +592,7 @@ class BaseGen(Dataset):
                 s.aux_mm, _ = arena.reserve(8 * _lib.MAX_AUX)
             for c, (key, vol) in enumerate(aux):
                 s.aux_src[c] = vol.data_ptr()
-                s.aux_raw[c] = raw_ws.data_ptr() + 4 * k_aux * N
+                s.aux_raw[c] = raw_ws.data_ptr() + 4 * k_aux * Np
                 s.aux_out[c] = aux_all[k_aux].data_ptr()
                 job['aux_out'][key] = aux_all[k_aux]
                 k_aux += 1

@@ -18,7 +18,7 @@ import torch
 from .. import _lib
 from ..draws import HostDraws
 from . import constants as K
-from .utils import DeformDict, DeformPlan, _stream
+from .utils import DeformDict, DeformPlan, _stream, scratch_stride
 
 
 def _ptr(t):
@@ -318,12 +318,13 @@ class NativePlanner:
         bufs.residual = res.data_ptr() if res is not None else None
         bufs.syn = syn_ws.data_ptr()
         bufs.syn_stride = src_pad
-        bufs.i_bf = ds._workspace('i_bf', total * N).data_ptr()
-        bufs.tmp = ds._workspace('tmp', total * 2 * N).data_ptr()
-        bufs.lowres = ds._workspace('lowres', total * N).data_ptr()
+        Np = scratch_stride(N)
+        bufs.i_bf = ds._workspace('i_bf', total * Np).data_ptr()
+        bufs.tmp = ds._workspace('tmp', total * 2 * Np).data_ptr()
+        bufs.lowres = ds._workspace('lowres', total * Np).data_ptr()
         if n_aux_total:
             bufs.aux_out = aux_all.data_ptr()
-            bufs.aux_raw = ds._workspace('aux_raw', n_aux_total * N).data_ptr()
+            bufs.aux_raw = ds._workspace('aux_raw', n_aux_total * Np).data_ptr()
         bufs.pair_ok = 1 if ds.pair_mode else 0
         if tr is not None:
             tr.append(('workspaces', _t.perf_counter()))
@@ -385,29 +386,30 @@ class NativePlanner:
             if 'syn_stride' in ds._ws:
                 syn_ws.zero_()
             ds._ws['syn_stride'] = src_pad
-        p_ibf = ds._workspace('i_bf', total * N).data_ptr()
-        p_tmp = ds._workspace('tmp', total * 2 * N).data_ptr()
-        p_low = ds._workspace('lowres', total * N).data_ptr()
-        p_raw = ds._workspace('aux_raw', n_aux_total * N).data_ptr() if n_aux_total else 0
+        Np = scratch_stride(N)
+        p_ibf = ds._workspace('i_bf', total * Np).data_ptr()
+        p_tmp = ds._workspace('tmp', total * 2 * Np).data_ptr()
+        p_low = ds._workspace('lowres', total * Np).data_ptr()
+        p_raw = ds._workspace('aux_raw', n_aux_total * Np).data_ptr() if n_aux_total else 0
         outs = (_lib.PlanOut * total)()
         o_np = np.frombuffer(outs, dtype=np.uint64).reshape(total, 9)
         q = np.arange(total, dtype=np.uint64)
-        step = np.uint64(4 * N)
+        step, pstep = np.uint64(4 * N), np.uint64(4 * Np)
         o_np[:, 0] = np.uint64(out.data_ptr()) + q * step
         o_np[:, 1] = (np.uint64(bfl.data_ptr()) + q * step) if want_bflog else 0
         o_np[:, 2] = (np.uint64(res.data_ptr()) + q * step) if want_res else 0
         o_np[:, 3] = np.uint64(syn_ws.data_ptr()) + q * np.uint64(4 * src_pad)
-        o_np[:, 4] = np.uint64(p_ibf) + q * step
-        o_np[:, 5] = np.uint64(p_tmp) + (2 * q) * step
-        o_np[:, 6] = np.uint64(p_tmp) + (2 * q + 1) * step
-        o_np[:, 7] = np.uint64(p_low) + q * step
+        o_np[:, 4] = np.uint64(p_ibf) + q * pstep
+        o_np[:, 5] = np.uint64(p_tmp) + (2 * q) * pstep
+        o_np[:, 6] = np.uint64(p_tmp) + (2 * q + 1) * pstep
+        o_np[:, 7] = np.uint64(p_low) + q * pstep
         o_np[:, 8] = 1 if ds.pair_mode else 0
         k_aux = 0
         for n in range(B):
             it = items[n]
             for c in range(it.n_aux):
                 it.aux_out[c] = aux_all.data_ptr() + 4 * N * k_aux
-                it.aux_raw[c] = p_raw + 4 * N * k_aux
+                it.aux_raw[c] = p_raw + 4 * Np * k_aux
                 k_aux += 1
         # ---- draws to replay (parity tests): scalars and small arrays flattened in log order
         keep = []

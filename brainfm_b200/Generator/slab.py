@@ -25,7 +25,7 @@ import torch.distributed as dist
 
 from .. import _lib, parallel as par
 from ..plan import band_host, resample_coords_host, zoom_tables_host
-from .utils import _stream
+from .utils import _stream, scratch_stride
 
 
 def _band_axis(x, axis, n_out, start, w, T, arena):
@@ -217,7 +217,7 @@ def _generate_slab_native(ds, native, idx, rank, world, group):
         mmf = torch.where(mm >= 0, mm, mm ^ 0x7fffffff).view(torch.float32)         # ord2f (csrc/common.cuh)
         keys = [k for k, _ in plan['metas'][0][5]]
         for a in range(n_aux):
-            raw = ds._ws['aux_raw'][a * N:(a + 1) * N].view(s0, s1, s2)[c0:c1]
+            raw = ds._ws['aux_raw'][a * scratch_stride(N):][:N].view(s0, s1, s2)[c0:c1]
             tgt = torch.empty((c1 - c0, s1, s2), dtype=torch.float32, device=dev)
             _lib.check(L.bfm_shift_scale_flip(raw.data_ptr(), tgt.data_ptr(), c1 - c0, s1 * s2,
                                               mmf[2 * a:2 * a + 1].data_ptr(), mmf[2 * a + 1:2 * a + 2].data_ptr(), 1.0,

@@ -20,6 +20,12 @@ def _stream():
     return C.c_void_p(torch._C._cuda_getCurrentRawStream(torch._C._cuda_getDevice()))
 
 
+def scratch_stride(N):
+    """Floats per sample slot of the fused chain's scratch (i_bf, tmp, lowres, aux_raw): N rounded up to a multiple of
+    4, so that every slot keeps the 16-byte alignment the 128-bit kernel paths need (include/bfm.h)."""
+    return (int(N) + 3) // 4 * 4
+
+
 def _need_cuda(t, what):
     if not isinstance(t, torch.Tensor) or not t.is_cuda:
         raise _lib.BfmError("%s must be a CUDA tensor: brainfm_b200 has no CPU path" % what)

@@ -1432,6 +1432,8 @@ __global__ void __launch_bounds__(256) k_gen_normalize(const bfm_gen_sample *__r
     }
 }
 
+static inline bool misaligned(const void *p, uintptr_t bytes) { return ((uintptr_t)p & (bytes - 1)) != 0; }
+
 static int check_batch(const bfm_gen_sample *h, const bfm_gen_sample *d, int B) {
     if (!h || !d || B <= 0) return fail(BFM_E_INVALID, "%s", "bfm_gen: null descriptors or empty batch");
     for (int b = 0; b < B; ++b) {
@@ -1454,6 +1456,17 @@ static int check_batch(const bfm_gen_sample *h, const bfm_gen_sample *d, int B) 
         if (s.n_band < 1 || s.n_band > 3) return fail(BFM_E_INVALID, "%s", "bfm_gen: n_band must be 1..3");
         if (s.d.size[0] != h[0].d.size[0] || s.d.size[1] != h[0].d.size[1] || s.d.size[2] != h[0].d.size[2])
             return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen: all samples of a batch share the output size");
+        // The kernels take 128-bit accesses without looking at the pointers: on the scratch whenever the low-res
+        // shape allows (k_gen_band<4>, k_gen_upsample), on the outputs whenever the output plane is a multiple of 4.
+        if (misaligned(s.i_bf, 16) || misaligned(s.tmp[0], 16) || misaligned(s.tmp[1], 16) ||
+            misaligned(s.lowres, 16) || misaligned(s.syn, 8))
+            return fail(BFM_E_INVALID, "%s", "bfm_gen: misaligned scratch (i_bf, tmp, lowres: 16 bytes; syn: 8)");
+        if ((((int64_t)s.d.size[1] * s.d.size[2]) & 3) == 0) {
+            bool bad = misaligned(s.out, 16) || misaligned(s.bflog_out, 16) || misaligned(s.residual, 16);
+            for (int a = 0; a < s.n_aux && a < BFM_MAX_AUX; ++a)
+                bad |= misaligned(s.aux_out[a], 16) || misaligned(s.aux_raw[a], 16);
+            if (bad) return fail(BFM_E_INVALID, "%s", "bfm_gen: misaligned output (16 bytes when size[1]*size[2] % 4 == 0)");
+        }
     }
     return BFM_OK;
 }

@@ -499,6 +499,7 @@ extern "C" int bfm_plan_run(const bfm_plan_cfg *cfg, int n_items, bfm_plan_item 
         return fail(BFM_E_INVALID, "%s", "bfm_plan_run: null buffer");
     const int ns = cfg->n_samples, total = n_items * ns;
     const int64_t N = (int64_t)cfg->size[0] * cfg->size[1] * cfg->size[2];
+    const int64_t Np = (N + 3) & ~(int64_t)3;        // scratch slots keep the 16-byte alignment of their base
     std::vector<bfm_plan_out> outs((size_t)total);
     for (int q = 0; q < total; ++q) {
         bfm_plan_out &o = outs[q];
@@ -506,10 +507,10 @@ extern "C" int bfm_plan_run(const bfm_plan_cfg *cfg, int n_items, bfm_plan_item 
         o.bflog_out = bufs->bflog_out ? bufs->bflog_out + q * N : nullptr;
         o.residual = bufs->residual ? bufs->residual + q * N : nullptr;
         o.syn = bufs->syn + q * bufs->syn_stride;
-        o.i_bf = bufs->i_bf + q * N;
-        o.tmp[0] = bufs->tmp + (2 * (int64_t)q) * N;
-        o.tmp[1] = bufs->tmp + (2 * (int64_t)q + 1) * N;
-        o.lowres = bufs->lowres + q * N;
+        o.i_bf = bufs->i_bf + q * Np;
+        o.tmp[0] = bufs->tmp + (2 * (int64_t)q) * Np;
+        o.tmp[1] = bufs->tmp + (2 * (int64_t)q + 1) * Np;
+        o.lowres = bufs->lowres + q * Np;
         o.syn_pair_ok = bufs->pair_ok;
     }
     int64_t k_aux = 0;
@@ -517,7 +518,7 @@ extern "C" int bfm_plan_run(const bfm_plan_cfg *cfg, int n_items, bfm_plan_item 
         for (int c = 0; c < items[n].n_aux && c < BFM_MAX_AUX; ++c) {
             if (!bufs->aux_out || !bufs->aux_raw) return fail(BFM_E_INVALID, "%s", "bfm_plan_run: null target buffer");
             items[n].aux_out[c] = bufs->aux_out + k_aux * N;
-            items[n].aux_raw[c] = bufs->aux_raw + k_aux * N;
+            items[n].aux_raw[c] = bufs->aux_raw + k_aux * Np;
             ++k_aux;
         }
     int64_t used = arena_used_in, upload = 0;

@@ -276,7 +276,11 @@ typedef struct bfm_gen_sample {
 } bfm_gen_sample;
 
 /* Each stage launches over samples [0,B).  `s_dev` is the device copy of the descriptor array,
- * `s_host` the host copy (grid sizing only). */
+ * `s_host` the host copy (grid sizing and argument checks only).
+ * Alignment (the kernels take 128-bit accesses without testing the pointers; every stage returns BFM_E_INVALID
+ * when one of these fails): i_bf, tmp[0], tmp[1] and lowres 16-byte aligned, syn 8-byte aligned, and when
+ * size[1]*size[2] % 4 == 0 also out, bflog_out, residual, aux_out[*] and aux_raw[*].  Per-sample scratch slots
+ * therefore advance by prod(size) rounded up to a multiple of 4 floats. */
 /* bfm_gen_plan: builds the banded blur-o-downsample tables flagged `build` on the device (no host work, no
  * host->device traffic for them); must precede bfm_gen_resample. */
 int bfm_gen_plan(const bfm_gen_sample *s_host, const bfm_gen_sample *s_dev, int B, void *stream);
@@ -385,9 +389,10 @@ int bfm_plan_batch(const bfm_plan_cfg *cfg, int n_items, const bfm_plan_item *it
                    int64_t *arena_used, int64_t *upload_bytes, bfm_gen_sample *descs_host, void **descs_dev,
                    bfm_plan_info *info, const double *replay, int64_t n_replay, int64_t *replay_used);
 
-/* Base pointers of a batch's buffers, per-sample strides implied: out / bflog_out / residual / i_bf / lowres advance by
- * prod(size) floats per sample, tmp by 2 * prod(size), syn by syn_stride; aux_out / aux_raw by prod(size) per fused
- * real-image target, in item order. */
+/* Base pointers of a batch's buffers, per-sample strides implied: out / bflog_out / residual advance by N = prod(size)
+ * floats per sample and aux_out by N per fused real-image target, in item order; the scratch advances by
+ * Npad = (N + 3) & ~3 floats (i_bf, lowres: Npad per sample, tmp: 2 * Npad, aux_raw: Npad per target) so that every
+ * slot keeps the 16-byte alignment of its base; syn by syn_stride. */
 typedef struct bfm_step_bufs {
     float *out, *bflog_out, *residual;
     float *syn;

@@ -104,8 +104,13 @@ CASES = {
 }
 
 
+def shape3(n):
+    """An int means a cube; a 3-tuple is taken as (x, y, z)."""
+    return tuple(int(v) for v in n) if isinstance(n, (tuple, list)) else (int(n),) * 3
+
+
 def build_volumes(src, kind, extra):
-    shp = (src, src, src)
+    shp = shape3(src)
     lab = ti.block_labels(shp) if kind == "block" else ti.brain_like_labels(shp)
     vols = {"Gen": lab, "T1": ti.smooth_image(shp, 0.0), "segmentation": ti.seg_labels(shp)}
     if "T2" in extra:
@@ -117,8 +122,8 @@ def build_volumes(src, kind, extra):
     if "registration" in extra:
         vols["registration"] = [ti.smooth_image(shp, 0.7 * i) * 50 for i in range(3)]
     if "mni" in extra:           # signed MNI-like coordinates: x < 0 on one side of a wavy mid-sagittal surface
-        ax = np.arange(src, dtype=np.float32) - (src - 1) / 2
-        base = [ax[:, None, None], ax[None, :, None], ax[None, None, :]]
+        ax = [np.arange(n, dtype=np.float32) - (n - 1) / 2 for n in shp]
+        base = [ax[0][:, None, None], ax[1][None, :, None], ax[2][None, None, :]]
         wob = [ti.smooth_image(shp, 0.7 * i) for i in range(3)]
         vols["registration"] = [(base[i] + 3 * (wob[i] - wob[i].mean()) / wob[i].std()).astype(np.float32)
                                 for i in range(3)]
@@ -128,15 +133,15 @@ def build_volumes(src, kind, extra):
 def cfg_for(size, over, option, ref):
     if ref:
         args = rs.load_generator_cfg()
-        base = ti.default_cfg((size,) * 3)
+        base = ti.default_cfg(shape3(size))
         for k, v in vars(base.task).items():
             setattr(args.task, k, v)
-        args.generator.size = [size] * 3
+        args.generator.size = list(shape3(size))
         args.mix_synth_prob = 0.0
         args.dataset_names = ["HCP"]
         args.modality_probs.HCP = ti.ns(T1=0., T2=0., FLAIR=0., CT=0., synth=1.)
     else:
-        args = ti.default_cfg((size,) * 3)
+        args = ti.default_cfg(shape3(size))
     args.dataset_option = option
     for k, v in over.items():
         node = args
@@ -183,7 +188,8 @@ def run_reference(name):
 
 
 def run_oracle(name):
-    size, src, kind, seed, over, extra, option, stride = CASES[name]
+    """name: a key of CASES or a case tuple of the same layout."""
+    size, src, kind, seed, over, extra, option, stride = CASES[name] if isinstance(name, str) else name
     vols = build_volumes(src, kind, extra)
     args = cfg_for(size, over, option, ref=False)
     orc = go.GeneratorOracle(args, vols, brain_id=(option == "brain_id"))

@@ -8,11 +8,11 @@ import pytest
 import torch
 
 from oracle import make_golden as mg
-from tests._harness import cuda_case, oracle_case, to_np
+from tests._harness import ATOL, RTOL, cuda_case, oracle_case, to_np
+from tests._harness import compare as _compare
 
 pytestmark = pytest.mark.gpu
 
-RTOL, ATOL = 1e-5, 1e-4
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 CASES = ["g64_s0", "g64_s1", "g64_s2", "g64_s3", "g64_s5_lowres", "g64_full_s4", "g160_s0", "g64_pathol_s7",
          "g64_pathol_s12", "g64_left_s9", "g64_ident_s23", "g64_realT1_s14", "g64_realT2_s15", "g64_realCT_s16"]
@@ -20,24 +20,6 @@ CASES = ["g64_s0", "g64_s1", "g64_s2", "g64_s3", "g64_s5_lowres", "g64_full_s4",
 # one-hots, cubic B-spline zoom back, random centre shift, CT contrast groups, PDE-advected pathology shapes
 CASES_R2 = ["g64_svf_s31", "g64_svf_s41", "g64_onehot_s43", "g64_onehot_s41", "g64_bspline_s43", "g64_bspline_s41",
             "g64_shift_s43", "g64_ct_s35", "g64_augpath_s47", "g64_augpath_s48"]
-
-
-def _compare(ref, got, name):
-    assert set(ref) == set(got), (name, sorted(set(ref) ^ set(got)))
-    report = {}
-    for k, a in ref.items():
-        b = got[k]
-        if not isinstance(a, torch.Tensor):
-            assert float(a) == float(b), (name, k)
-            continue
-        a, b = to_np(a), to_np(b)
-        assert a.shape == b.shape, (name, k, a.shape, b.shape)
-        if "segmentation" in k and np.all((a == 0) | (a == 1)):
-            assert np.array_equal(a, b), "%s %s: one-hot differs in %d voxels" % (name, k, int((a != b).sum()))
-        else:
-            np.testing.assert_allclose(b, a, rtol=RTOL, atol=ATOL, err_msg="%s %s" % (name, k))
-        report[k] = float(np.abs(a.astype(np.float64) - b).max())
-    return report
 
 
 @pytest.mark.parametrize("name", CASES + CASES_R2)

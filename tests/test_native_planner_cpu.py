@@ -13,6 +13,7 @@ from brainfm_b200 import _lib
 from brainfm_b200.Generator import constants as K
 from oracle import make_golden as mg
 from tests._harness import oracle_case
+from tests.test_chain_shapes_gpu import CASES as SHAPE_CASES
 
 FAKE = 0x7f0000000000          # "device" addresses: never dereferenced by the planner
 
@@ -89,16 +90,21 @@ def flatten_log(log):
     return np.ascontiguousarray(np.concatenate(vals))
 
 
-@pytest.mark.parametrize("name", ["g64_s0", "g64_s1", "g64_s2", "g64_s3", "g64_s5_lowres", "g160_s0"])
+# the odd and anisotropic grids of test_chain_shapes_gpu that the library plans (one sample per item, no mixing)
+ODD = [k for k, v in SHAPE_CASES.items() if v[6] == "default" and "mix_synth_prob" not in v[4]]
+
+
+@pytest.mark.parametrize("name", ["g64_s0", "g64_s1", "g64_s2", "g64_s3", "g64_s5_lowres", "g160_s0"] + ODD)
 def test_replay_reproduces_the_oracle_setup(name):
-    size, src, kind, seed, over, extra, option, stride = mg.CASES[name]
-    item, orc = oracle_case(name)
+    case = mg.CASES.get(name) or SHAPE_CASES[name]
+    size, src, kind, seed, over, extra, option, stride = case
+    item, orc = oracle_case(case)
     args = mg.cfg_for(size, over, option, ref=False)
     gen = dict(vars(args.generator))
     gen.update(vars(args.synth_image_generator))
-    cfg, keep = make_cfg([size] * 3, args.generator, aug_sets=[gen])
+    cfg, keep = make_cfg(list(mg.shape3(size)), args.generator, aug_sets=[gen])
     flat = flatten_log(orc.log)
-    r = plan(cfg, 1, [src] * 3, replay=flat)
+    r = plan(cfg, 1, list(mg.shape3(src)), replay=flat)
     assert r['consumed'] == flat.size
     inf, s = r['info'][0], r['descs'][0]
     st = orc.setups
@@ -238,3 +244,26 @@ def test_real_input_modes_are_drawn_like_read_input():
             else:
                 assert inf.input_mode == 0 and s.bfsmall
     assert 0.8 < n_ct / 160 < 0.98
+
+
+@pytest.mark.parametrize("field", ["lowres", "tmp1", "i_bf", "syn", "out"])
+def test_misaligned_buffers_are_refused_before_any_launch(field):
+    """Every stage's argument check: the kernels take 128-bit accesses on the scratch (and on the outputs of a plane
+    that is a multiple of 4) without testing the pointers, so a misaligned slot must come back as BFM_E_INVALID.  The
+    descriptor is planned with (aligned) fake device addresses and then broken in exactly one field, so the check
+    returns before anything is launched."""
+    args = mg.cfg_for(64, {}, "default", ref=False)
+    gen = dict(vars(args.generator))
+    gen.update(vars(args.synth_image_generator))
+    cfg, keep = make_cfg([64] * 3, args.generator, aug_sets=[gen])
+    r = plan(cfg, 1, [96] * 3, seed=4)
+    s = r['descs'][0]
+    if field == "tmp1":                       # one float off: misaligned for 16-byte and for 8-byte slots
+        s.tmp[1] = FAKE + 4
+    else:
+        setattr(s, field, FAKE + 4)
+    L = _lib.lib()
+    for stage in (L.bfm_gen_run, L.bfm_gen_plan, L.bfm_gen_bbox, L.bfm_gen_gmm, L.bfm_gen_warp, L.bfm_gen_resample,
+                  L.bfm_gen_finish):
+        assert stage(C.addressof(r['descs']), FAKE, 1, None) == _lib.BFM_E_INVALID
+        assert "misaligned" in L.bfm_last_error().decode()

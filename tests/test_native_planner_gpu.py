@@ -8,8 +8,8 @@ import pytest
 import torch
 
 from oracle import make_golden as mg
+from tests._harness import compare as _compare
 from tests._harness import cuda_case, oracle_case, to_np
-from tests.test_gen_parity_gpu import _compare
 
 pytestmark = pytest.mark.gpu
 
