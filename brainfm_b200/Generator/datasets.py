@@ -393,9 +393,8 @@ class BaseGen(Dataset):
     # ---- host-side plan of one synthetic sample (all scalar draws, reference order) ----------------
     def _stock_chain(self, input_mode):
         steps = self.augmentation_steps['synth'] if input_mode == 'synth' else self.augmentation_steps['real']
-        return (list(steps) == _STOCK_STEPS and all(K.augmentation_funcs.get(k) is K._STOCK_AUGMENTATION[k]
-                                                    for k in _STOCK_STEPS)
-                and not self.synth_args.bspline_zooming)
+        return list(steps) == _STOCK_STEPS and all(K.augmentation_funcs.get(k) is K._STOCK_AUGMENTATION[k]
+                                                   for k in _STOCK_STEPS)
 
     def _plan_synth(self, setups, target, arena=None, real=False):
         """Draws of generate_sample + the stock augmentation chain, in the reference's order
@@ -539,6 +538,7 @@ class BaseGen(Dataset):
                 sample['bias_field_log'] = bfl_all[k_bfl]
                 k_bfl += 1
             s.flip = 1 if job['flip'] else 0
+            s.zoom_order = 3 if self.synth_args.bspline_zooming else 0
             # resolution degradation: banded passes in ascending factor order, identity axes folded away
             new = [int(v) for v in p['new_size']]
             order = sorted(range(3), key=lambda a: new[a] / size[a])

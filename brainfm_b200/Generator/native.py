@@ -53,7 +53,8 @@ class NativePlanner:
         changed gen_args since (curricula, update_gen_args with new values)."""
         ds = self.ds
         a = ds.synth_args
-        fp = [getattr(a, k) for k in self._KEYS] + [ds.gen_args.mix_synth_prob, tuple(ds.size)]
+        fp = [getattr(a, k) for k in self._KEYS] + [getattr(a, 'bspline_zooming', False), ds.gen_args.mix_synth_prob,
+                                                    tuple(ds.size)]
         for mode in ('synth', 'T1'):
             for overrides in ds._gen_arg_sets(mode):
                 for o in overrides:
@@ -72,7 +73,7 @@ class NativePlanner:
     @staticmethod
     def config_ok(ds):
         a = ds.synth_args
-        if a.left_hemis_only or a.random_shift or getattr(a, 'bspline_zooming', False):
+        if a.left_hemis_only or a.random_shift:
             return False
         if ds.gen_args.mix_synth_prob > 0 or 'surface' in ds.tasks or 'pathology' in ds.tasks:
             return False
@@ -103,6 +104,7 @@ class NativePlanner:
         cfg.size[:] = size
         cfg.res[:] = [float(v) for v in ds.res_training_data]
         cfg.low_res_only = int(bool(a.low_res_only))
+        cfg.bspline_zooming = int(bool(getattr(a, 'bspline_zooming', False)))
         cfg.nonlinear_transform = int(bool(a.nonlinear_transform))
         for k in ('photo_prob', 'pathology_prob', 'random_shape_prob', 'flip_prob', 'max_rotation', 'max_shear',
                   'max_scaling', 'nonlin_scale_min', 'nonlin_scale_max', 'nonlin_std_max', 'ct_prob'):

@@ -236,6 +236,9 @@ def generate_slab(ds, idx, rank=None, world=None, group=None):
         rank = dist.get_rank(group) if dist.is_initialized() else 0
     if world is None:
         world = dist.get_world_size(group) if dist.is_initialized() else 1
+    if getattr(ds.synth_args, 'bspline_zooming', False):
+        # the cubic zoom's dct2 prefilter is a recursion along the whole x axis: no fixed halo covers it
+        raise NotImplementedError("slab mode does not cover bspline_zooming")
     ds.cache.begin_batch()
     native = ds._native_planner([idx]) if not getattr(ds.rng, 'replay', False) else None
     if native is not None and native.n_samples == 1:

@@ -47,7 +47,7 @@ class GenSample(C.Structure):
                 ("n_aux", c_i), ("aux_src", c_p * MAX_AUX), ("aux_raw", c_p * MAX_AUX), ("aux_out", c_p * MAX_AUX),
                 ("aux_mm", c_p), ("x_begin", c_i), ("x_count", c_i),
                 ("gen_small", c_i), ("fs_std", c_f), ("bf_std", c_f), ("real_input", c_i), ("syn_pair_ok", c_i),
-                ("gmm_xr", c_p)]
+                ("zoom_order", c_i), ("gmm_xr", c_p)]
 
 
 # ---- native host planner (bfm_plan_batch) ----------------------------------------------------------------
@@ -70,6 +70,7 @@ class PlanCfg(C.Structure):
                 ("max_rotation", c_d), ("max_shear", c_d), ("max_scaling", c_d),
                 ("nonlin_scale_min", c_d), ("nonlin_scale_max", c_d), ("nonlin_std_max", c_d),
                 ("ct_prob", c_d), ("mix_synth_prob", c_d), ("ct_group", C.c_int8 * 256), ("n_samples", c_i),
+                ("bspline_zooming", c_i),
                 ("aug", PlanAug * PLAN_MAX_SAMPLES), ("aug_real", PlanAug * PLAN_MAX_SAMPLES),
                 ("fwd", c_p * 3), ("inv", c_p * 3), ("ends", c_p * 3), ("ident_start", c_p), ("ident_w", c_p)]
 
@@ -131,6 +132,7 @@ _PROTOS = {
     "bfm_gen_warp": (c_i, [c_p, c_p, c_i, c_p]),
     "bfm_gen_resample": (c_i, [c_p, c_p, c_i, c_p]),
     "bfm_gen_finish": (c_i, [c_p, c_p, c_i, c_p]),
+    "bfm_gen_zoom_coords": (c_i, [c_i, c_i, c_p, c_p]),
     "bfm_gen_run": (c_i, [c_p, c_p, c_i, c_p]),
     "bfm_plan_batch": (c_i, [c_p, c_i, c_p, c_p, c_u64, c_u64, c_p, c_p, c_i64, C.POINTER(c_i64), C.POINTER(c_i64),
                              c_p, C.POINTER(c_p), c_p, c_p, c_i64, C.POINTER(c_i64)]),

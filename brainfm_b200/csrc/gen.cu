@@ -10,12 +10,13 @@
 //   warp     coordinates -> trilinear gather of syn -> mix -> clamp -> gamma -> bias field
 //            (utils.py:140-192, datasets.py:379-411, utils.py:568-589) -> i_bf, bflog_out
 //   resample blur o downsample as banded per-axis maps + noise (utils.py:83-94, 591-609, 633-638)
-//   finish   myzoom_torch back to the grid, global max, normalise, flip (datasets.py:337-352)
+//   finish   myzoom_torch (or, with bspline_zooming, the cubic B-spline resize) back to the grid, global max,
+//            normalise, flip (datasets.py:337-352)
 //
 // Every kernel is instruction-issue bound on B200 (see profiles/), so the code is organised to minimise
 // instructions per voxel: the sample descriptor is staged in shared memory, loop invariants live in registers,
 // a warp owns several rows so per-k table entries are loaded once, element indices are 32-bit.
-#include "common.cuh"
+#include "spline.cuh"
 
 namespace bfm {
 
@@ -27,6 +28,22 @@ constexpr int kPkNodes = 48;         // z nodes (+1 duplicate of the last) of a 
 __host__ __device__ __forceinline__ bool use_pairs(const bfm_gen_sample &s) {
     return s.syn_pair_ok && s.n_aux == 1 && !s.mix[0] && !s.real_input && !(s.d.src[2] & 3) && !s.d.F_full &&
            (!s.d.fsmall || s.d.fs[2] < kPkNodes) && (!s.bfsmall || s.bs[2] < kPkNodes);
+}
+
+// Undegraded resolution class (resolution == thickness == the training resolution: identity band, new_size == size):
+// the banded pass is a copy and the zoom back is the identity (weights exactly 1 and 0), so those samples take
+// k_gen_identity -- noise + clamp straight from i_bf into `out` -- instead of the band and upsample kernels.
+__host__ __device__ __forceinline__ bool is_identity_sample(const bfm_gen_sample &s) {
+    return s.n_band == 1 && s.band[0].T == 1 && s.band[0].build == 0 && s.x_count == 0 &&
+           s.new_size[0] == s.d.size[0] && s.new_size[1] == s.d.size[1] && s.new_size[2] == s.d.size[2] &&
+           ((s.d.size[1] * s.d.size[2]) & 3) == 0;
+}
+
+// Cubic zoom back (zoom_order == 3, the generator's bspline_zooming): prefilter + cubic pull in the finish stage.  The
+// undegraded class keeps k_gen_identity: at integer nodes the cubic pull of the prefiltered coefficients reproduces
+// its input up to rounding.
+__host__ __device__ __forceinline__ bool cubic_zoom(const bfm_gen_sample &s) {
+    return s.zoom_order == 3 && !is_identity_sample(s);
 }
 
 __device__ __forceinline__ void stage_desc(bfm_gen_sample *dst, const bfm_gen_sample *src) {
@@ -51,7 +68,12 @@ __global__ void k_gen_bbox_init(const bfm_gen_sample *__restrict__ S) {
         else if (threadIdx.x < 6) bb[threadIdx.x] = 0;
         else if (threadIdx.x == 6) bb[6] = 1;               // 1 = full scan still required
     }
-    if (threadIdx.x == 7) *S[blockIdx.x].maxval = 0.f;      // chain values are >= 0 after the noise clamp
+    if (threadIdx.x == 7) {
+        // chain values are >= 0 after the noise clamp and the linear zoom keeps them so: the raw bits order them.  The
+        // cubic zoom overshoots below 0 next to clamped zeros: order-preserving encoding from -inf (k_gen_cubic_zoom).
+        if (cubic_zoom(S[blockIdx.x])) *(int *)S[blockIdx.x].maxval = f2ord(-INFINITY);
+        else *S[blockIdx.x].maxval = 0.f;
+    }
     if (threadIdx.x >= 8 && threadIdx.x < 8 + 2 * S[blockIdx.x].n_aux) {
         const int q = threadIdx.x - 8;
         S[blockIdx.x].aux_mm[q] = (q & 1) ? f2ord(-INFINITY) : f2ord(INFINITY);
@@ -1054,15 +1076,6 @@ k_gen_warp_pk(const bfm_gen_sample *__restrict__ S, const __grid_constant__ PkPa
     else warp_rows_pk<0>(sh, t1F, t1B, rpb, P.s[blockIdx.z], P.one);
 }
 
-// Undegraded resolution class (resolution == thickness == the training resolution: identity band, new_size == size):
-// the banded pass is a copy and the zoom back is the identity (weights exactly 1 and 0), so those samples take
-// k_gen_identity -- noise + clamp straight from i_bf into `out` -- instead of the band and upsample kernels.
-__host__ __device__ __forceinline__ bool is_identity_sample(const bfm_gen_sample &s) {
-    return s.n_band == 1 && s.band[0].T == 1 && s.band[0].build == 0 && s.x_count == 0 &&
-           s.new_size[0] == s.d.size[0] && s.new_size[1] == s.d.size[1] && s.new_size[2] == s.d.size[2] &&
-           ((s.d.size[1] * s.d.size[2]) & 3) == 0;
-}
-
 // ---------------------------------------------------------------------------------------------- resample
 // One banded pass.  Axis 0/1: a thread owns VEC consecutive z outputs (128-bit loads when VEC == 4); the tap
 // weight is uniform across the warp.  Axis 2: a thread owns one output, taps are contiguous.
@@ -1333,6 +1346,7 @@ __global__ void __launch_bounds__(160, UPS_MINB) k_gen_upsample(const bfm_gen_sa
     const int s0 = s.d.size[0], s1 = s.d.size[1], s2 = s.d.size[2];
     if ((int)blockIdx.y >= s0 || (int)blockIdx.x * kUR >= s1) return;
     if (is_identity_sample(s)) return;                  // k_gen_identity (resample stage) already wrote `out`
+    if (cubic_zoom(s)) return;                          // k_gen_cubic_zoom
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nwarps = blockDim.x >> 5;
     const int ly = s.new_size[1], lz = s.new_size[2];
     const int i = blockIdx.y, j0 = blockIdx.x * kUR, j1 = min(j0 + kUR, s1);
@@ -1390,6 +1404,214 @@ __global__ void __launch_bounds__(160, UPS_MINB) k_gen_upsample(const bfm_gen_sa
     }
 }
 
+// ---------------------------------------------------------------------------------------------- cubic zoom back
+// bspline_zooming (datasets.py:337-338): interpol.resize(I, shape=size, anchor='edge', interpolation=3, bound='dct2',
+// prefilter=True) of `lowres` back to the training grid.  Three prefilter launches (one per axis, in place on
+// `lowres`, which is dead after this stage), then k_gen_cubic_zoom.  blockIdx.z = sample throughout.
+constexpr int kCubicLines = 32;   // lines per block of the tiled z prefilter
+
+// the prefilter of one axis of length n: cubic B-spline (one pole, sqrt(3) - 2), dct2 boundary -- the arguments
+// brainfm_b200.interpol.spline_coeff passes to bfm_spline_filter
+__device__ __forceinline__ FilterArgs cubic_filter_args(int n) {
+    FilterArgs a;
+    a.outer = 1; a.inner = 1; a.n = n; a.bound = 3; a.npoles = 1;
+    a.poles[0] = sqrt(3.0) - 2.0; a.poles[1] = a.poles[2] = 0.0;
+    return a;
+}
+
+// Sample coordinate of output o of an edge-anchored resize from n_in to n_out (interpol resize, anchor='edge':
+// torch.arange(n_out) * scale + 0.5 * (scale - 1) with scale = n_in / n_out): a float32 product and a float32 sum,
+// the Python floats rounded to float32 first.
+__device__ __forceinline__ float edge_coord(int o, int n_in, int n_out) {
+    const double scale = (double)n_in / (double)n_out;
+    return __fadd_rn(__fmul_rn((float)o, (float)scale), (float)(0.5 * (scale - 1.0)));
+}
+
+// The 4 taps of a cubic pull at x with dct2 folding: k_pull_fast's node indices and weights (the dct2 sign is 1).
+__device__ __forceinline__ void cubic_taps(float x, int n, int idx[4], float w[4]) {
+    const float f0 = floorf(x - 1.f);
+    const float dist0 = x - f0;
+    const int i0 = (int)f0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        idx[k] = bound_index_t<int>(3, i0 + k, n);
+        w[k] = spline_weight<float>(3, dist0 - float(k));
+    }
+}
+
+// Prefilter along x (AXIS 0) or y (AXIS 1): one thread per line, adjacent threads on adjacent lines (adjacent z, so
+// every step of the recursion is a coalesced access); filter_line of bfm_spline_filter, with its dct2 weight table
+// in shared memory.  A length-1 line is its own coefficient (bfm_spline_filter returns before any launch then).
+template <int AXIS>
+__global__ void __launch_bounds__(256) k_gen_prefilter(const bfm_gen_sample *__restrict__ S) {
+    extern __shared__ float wt[];
+    const bfm_gen_sample &s = S[blockIdx.z];
+    if (!cubic_zoom(s)) return;
+    const int l0 = s.new_size[0], l1 = s.new_size[1], l2 = s.new_size[2];
+    const int n = AXIS == 0 ? l0 : l1;
+    const int lines = AXIS == 0 ? l1 * l2 : l0 * l2;
+    if (n == 1 || (int)(blockIdx.x * blockDim.x) >= lines) return;
+    const FilterArgs a = cubic_filter_args(n);
+    for (int e = threadIdx.x; e < n; e += blockDim.x) wt[e] = filter_weight(a, e);
+    __syncthreads();
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= lines) return;
+    const int x = AXIS == 0 ? 0 : q / l2, z = q - x * l2;     // AXIS 0: q = y * l2 + z
+    filter_line<float, int>(s.lowres + (size_t)x * l1 * l2 + z, AXIS == 0 ? l1 * l2 : l2, a, wt);
+}
+
+// Prefilter along z: the lines are contiguous, so a block stages kCubicLines of them in shared memory with coalesced
+// loads (128-bit when the line length is a multiple of 4), one thread per line runs the recursion there (odd pitch:
+// conflict free) and the tile is written back once -- k_spline_filter_tile<true> batched over descriptors.
+__global__ void __launch_bounds__(128) k_gen_prefilter_z(const bfm_gen_sample *__restrict__ S) {
+    extern __shared__ float tile[];
+    const bfm_gen_sample &s = S[blockIdx.z];
+    if (!cubic_zoom(s)) return;
+    const int n = s.new_size[2], rows = s.new_size[0] * s.new_size[1];
+    const int r0 = blockIdx.x * kCubicLines;
+    if (n == 1 || r0 >= rows) return;
+    const int tid = threadIdx.x, pitch = n | 1, nl = min(kCubicLines, rows - r0), total = nl * n;
+    float *wt = tile + kCubicLines * pitch;
+    const FilterArgs a = cubic_filter_args(n);
+    for (int e = tid; e < n; e += blockDim.x) wt[e] = filter_weight(a, e);
+    float *base = s.lowres + (size_t)r0 * n;
+    if ((n & 3) == 0) {                                 // rows start on multiples of 4 floats of a 16-byte aligned base
+        for (int e = 4 * tid; e < total; e += 4 * blockDim.x) {
+            const float4 v = *(const float4 *)(base + e);
+            const int row = e / n;
+            float *t = tile + row * pitch + (e - row * n);
+            t[0] = v.x; t[1] = v.y; t[2] = v.z; t[3] = v.w;
+        }
+    } else {
+        for (int e = tid; e < total; e += blockDim.x) {
+            const int row = e / n;
+            tile[row * pitch + (e - row * n)] = base[e];
+        }
+    }
+    __syncthreads();
+    if (tid < nl) filter_line<float, int>(tile + tid * pitch, 1, a, wt);
+    __syncthreads();
+    if ((n & 3) == 0) {
+        for (int e = 4 * tid; e < total; e += 4 * blockDim.x) {
+            const int row = e / n;
+            const float *t = tile + row * pitch + (e - row * n);
+            *(float4 *)(base + e) = make_float4(t[0], t[1], t[2], t[3]);
+        }
+    } else {
+        for (int e = tid; e < total; e += blockDim.x) {
+            const int row = e / n;
+            base[e] = tile[row * pitch + (e - row * n)];
+        }
+    }
+}
+
+// Cubic pull of the prefiltered `lowres` at the edge-anchored coordinates, evaluated separably in k_gen_upsample's
+// layout: block = (x plane i, kUR output rows), thread = k.  The axis-0 pass (4 taps along x) of the low-res rows
+// under the block's rows goes to shared memory (t1), then the axis-1 pass of each output row (t2), then 4 taps along
+// z per voxel.  The reference sums the 64 taps of a voxel in one loop; the separable sums round in another order
+// (float32 differences of a few ulp).  Stores the UNNORMALISED value at its final (flipped) position and reduces the
+// maximum with the order-preserving encoding: the cubic output can be negative.
+// ny_cap: low-res rows of t1 the host sized the shared memory for (>= the rows any block touches).
+__global__ void __launch_bounds__(160) k_gen_cubic_zoom(const bfm_gen_sample *__restrict__ S, int ny_cap) {
+    extern __shared__ float smem[];
+    __shared__ float red[8];
+    __shared__ int yi_s[kUR][4];
+    __shared__ float yw_s[kUR][4];
+    const bfm_gen_sample &s = S[blockIdx.z];
+    const int s0 = s.d.size[0], s1 = s.d.size[1], s2 = s.d.size[2];
+    if ((int)blockIdx.y >= s0 || (int)blockIdx.x * kUR >= s1) return;
+    if (!cubic_zoom(s)) return;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nwarps = blockDim.x >> 5;
+    const int lx = s.new_size[0], ly = s.new_size[1], lz = s.new_size[2];
+    const int i = blockIdx.y, j0 = blockIdx.x * kUR, nr = min(kUR, s1 - j0);
+    // low-res rows under output rows j0 .. j0+nr-1: the first node of a row is monotone in j, and dct2 folds the
+    // taps of the edge rows back inside [max(0, first node of j0), min(ly - 1, first node of the last row + 3)]
+    const int y0 = max(0, (int)floorf(edge_coord(j0, ly, s1) - 1.f));
+    const int y1 = min(ly - 1, (int)floorf(edge_coord(j0 + nr - 1, ly, s1) - 1.f) + 3);
+    const int ny = y1 - y0 + 1;
+    float *t1 = smem;                                   // [ny_cap][lz]: axis-0 pass at this i
+    float *t2 = smem + (size_t)ny_cap * lz;             // [kUR][lz]:    axis-1 pass of the block's rows
+    {
+        int xi[4];
+        float xw[4];
+        cubic_taps(edge_coord(i, lx, s0), lx, xi, xw);
+        const float *src[4];
+#pragma unroll
+        for (int t = 0; t < 4; ++t) src[t] = s.lowres + ((size_t)xi[t] * ly + y0) * lz;
+        const int n = ny * lz;                          // rows y0..y1 are contiguous in the low-res volume
+        if ((lz & 3) == 0) {                            // 128-bit loads: every row block starts on a multiple of lz
+            float4 *t4 = (float4 *)t1;
+            for (int q = tid; q < (n >> 2); q += blockDim.x) {
+                float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+                for (int t = 0; t < 4; ++t) {
+                    const float4 v = __ldg((const float4 *)src[t] + q);
+                    acc.x = fmaf(v.x, xw[t], acc.x); acc.y = fmaf(v.y, xw[t], acc.y);
+                    acc.z = fmaf(v.z, xw[t], acc.z); acc.w = fmaf(v.w, xw[t], acc.w);
+                }
+                t4[q] = acc;
+            }
+        } else {
+            for (int q = tid; q < n; q += blockDim.x) {
+                float acc = 0.f;
+#pragma unroll
+                for (int t = 0; t < 4; ++t) acc = fmaf(__ldg(src[t] + q), xw[t], acc);
+                t1[q] = acc;
+            }
+        }
+    }
+    if (tid < nr) {
+        int yi[4];
+        float yw[4];
+        cubic_taps(edge_coord(j0 + tid, ly, s1), ly, yi, yw);
+#pragma unroll
+        for (int t = 0; t < 4; ++t) { yi_s[tid][t] = (yi[t] - y0) * lz; yw_s[tid][t] = yw[t]; }
+    }
+    __syncthreads();
+    for (int r = 0; r < nr; ++r) {
+        const int a0 = yi_s[r][0], a1 = yi_s[r][1], a2 = yi_s[r][2], a3 = yi_s[r][3];
+        const float w0 = yw_s[r][0], w1 = yw_s[r][1], w2 = yw_s[r][2], w3 = yw_s[r][3];
+        for (int z = tid; z < lz; z += blockDim.x) {
+            float acc = fmaf(t1[a0 + z], w0, 0.f);
+            acc = fmaf(t1[a1 + z], w1, acc);
+            acc = fmaf(t1[a2 + z], w2, acc);
+            t2[r * lz + z] = fmaf(t1[a3 + z], w3, acc);
+        }
+    }
+    __syncthreads();
+    const int plane_out = (s.flip ? s0 - 1 - i : i) * s1;
+    float hi = -INFINITY;
+    for (int k = tid; k < s2; k += blockDim.x) {
+        int zi[4];
+        float zw[4];
+        cubic_taps(edge_coord(k, lz, s2), lz, zi, zw);
+        float *__restrict__ o = s.out + (size_t)(plane_out + j0) * s2 + k;
+#pragma unroll 4
+        for (int r = 0; r < nr; ++r) {
+            const float *t = t2 + r * lz;
+            float acc = fmaf(t[zi[0]], zw[0], 0.f);
+            acc = fmaf(t[zi[1]], zw[1], acc);
+            acc = fmaf(t[zi[2]], zw[2], acc);
+            acc = fmaf(t[zi[3]], zw[3], acc);
+            o[(size_t)r * s2] = acc;
+            hi = fmaxf(hi, acc);
+        }
+    }
+    hi = warp_max(hi);
+    if (lane == 0) red[warp] = hi;
+    __syncthreads();
+    if (tid == 0) {
+        for (int w = 1; w < nwarps; ++w) hi = fmaxf(hi, red[w]);
+        atomicMax((int *)s.maxval, f2ord(hi));
+    }
+}
+
+// edge_coord for o = 0 .. n_out-1 (bfm_gen_zoom_coords)
+__global__ void k_gen_zoom_coords(int n_in, int n_out, float *out) {
+    const int o = blockIdx.x * blockDim.x + threadIdx.x;
+    if (o < n_out) out[o] = edge_coord(o, n_in, n_out);
+}
+
 // I / max(I), optional high_res_residual (datasets.py:342-347) and the real-image targets'
 // `Idef -= min; Idef /= max; flip` (utils.py:326-329).  One thread = VEC consecutive z voxels of one x plane.
 template <int VEC>
@@ -1404,7 +1626,7 @@ __global__ void __launch_bounds__(256) k_gen_normalize(const bfm_gen_sample *__r
     const int io = s.flip ? s0 - 1 - i : i;
     const size_t pin = (size_t)i * plane + q, pout = (size_t)io * plane + q;
     // I / max(I) as a multiplication by the correctly rounded reciprocal: <= 1 ulp from the division
-    const float rmx = __frcp_rn(*s.maxval);
+    const float rmx = __frcp_rn(cubic_zoom(s) ? ord2f(*(const int *)s.maxval) : *s.maxval);
     float y[VEC];
     if (VEC == 4) {
         const float4 v = *(const float4 *)(s.out + pout);
@@ -1454,6 +1676,7 @@ static int check_batch(const bfm_gen_sample *h, const bfm_gen_sample *d, int B) 
         if (s.real_input && s.mix[0])
             return fail(BFM_E_INVALID, "%s", "bfm_gen: real-image inputs are not mixed");
         if (s.n_band < 1 || s.n_band > 3) return fail(BFM_E_INVALID, "%s", "bfm_gen: n_band must be 1..3");
+        if (s.zoom_order != 0 && s.zoom_order != 3) return fail(BFM_E_INVALID, "%s", "bfm_gen: zoom_order must be 0 or 3");
         if (s.d.size[0] != h[0].d.size[0] || s.d.size[1] != h[0].d.size[1] || s.d.size[2] != h[0].d.size[2])
             return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen: all samples of a batch share the output size");
         // The kernels take 128-bit accesses without looking at the pointers: on the scratch whenever the low-res
@@ -1756,9 +1979,23 @@ int bfm_gen_finish(const bfm_gen_sample *h, const bfm_gen_sample *d, int B, void
     int rc = check_batch(h, d, B);
     if (rc) return rc;
     int lz = 1, ny = 1, s0 = 0, s1 = 0, s2 = 0;
-    bool vec = false, scalar = false;
+    bool vec = false, scalar = false, linear = false;
+    int c_lz = 0, c_ny = 1, c_n0 = 1, c_n1 = 1;          // cubic zoom: line lengths and low-res rows under kUR rows
+    int64_t c_lines0 = 0, c_lines1 = 0, c_rows2 = 0;     // lines of the x, y and z prefilter
     for (int b = 0; b < B; ++b) {
         const bfm_gen_sample &s = h[b];
+        if (cubic_zoom(s)) {
+            const int *l = s.new_size;
+            c_lz = max(c_lz, l[2]); c_n0 = max(c_n0, l[0]); c_n1 = max(c_n1, l[1]);
+            c_lines0 = max(c_lines0, (int64_t)l[1] * l[2]);
+            c_lines1 = max(c_lines1, (int64_t)l[0] * l[2]);
+            c_rows2 = max(c_rows2, (int64_t)l[0] * l[1]);
+            // the first nodes of kUR consecutive rows span <= kUR * ly / s1 + 1 low-res rows (+1 for the float32
+            // coordinates), plus 3 more taps; checked exhaustively for ly, s1 <= 320
+            c_ny = max(c_ny, min(l[1], (int)((int64_t)kUR * l[1] / s.d.size[1]) + 8));
+        } else {
+            linear = true;
+        }
         lz = max(lz, s.new_size[2]);
         // low-res rows under kUR output rows: at most kUR * ly / s1 + 2 (and never more than ly)
         const int rows = min(s.new_size[1], (int)((int64_t)kUR * s.new_size[1] / s.d.size[1]) + 3);
@@ -1769,14 +2006,38 @@ int bfm_gen_finish(const bfm_gen_sample *h, const bfm_gen_sample *d, int B, void
     const size_t smem = (size_t)ny * lz * sizeof(float);
     if (smem > 200 * 1024) return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen_finish: low-res rows too long for shared memory");
     if (s0 > 65535 || B > 65535) return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen_finish: grid too large");
-    if (smem > 40 * 1024)
-        cudaFuncSetAttribute(k_gen_upsample, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     cudaStream_t st = (cudaStream_t)stream;
     const int threads = min(160, (s2 + 31) / 32 * 32);
     const int64_t plane = (int64_t)s1 * s2;
-    k_gen_upsample<<<dim3((s1 + kUR - 1) / kUR, s0, B), threads, smem, st>>>(d, lz, ny);
-    rc = check_launch("bfm_gen_finish");
-    if (rc) return rc;
+    if (c_lz > 0) {
+        const size_t smem_z = ((size_t)kCubicLines * (c_lz | 1) + c_lz) * sizeof(float);
+        const size_t smem_c = (size_t)(c_ny + kUR) * c_lz * sizeof(float);
+        if (smem_z > 200 * 1024 || smem_c > 200 * 1024 || (c_n0 > c_n1 ? c_n0 : c_n1) > 12 * 1024)
+            return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen_finish: low-res volume too large for the cubic zoom");
+        if (c_lines0 > (1LL << 30) || c_lines1 > (1LL << 30) || c_rows2 > (1LL << 30))
+            return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen_finish: grid too large");
+        // without the opt-in, static + dynamic shared memory must fit 48 KB (k_gen_cubic_zoom has ~1 KB static):
+        // opt in from 40 KB, as k_gen_upsample does
+        if (smem_z > 40 * 1024)
+            cudaFuncSetAttribute(k_gen_prefilter_z, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_z);
+        if (smem_c > 40 * 1024)
+            cudaFuncSetAttribute(k_gen_cubic_zoom, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_c);
+        k_gen_prefilter<0><<<dim3((unsigned)((c_lines0 + 255) / 256), 1, B), 256, c_n0 * sizeof(float), st>>>(d);
+        if ((rc = check_launch("bfm_gen_finish"))) return rc;
+        k_gen_prefilter<1><<<dim3((unsigned)((c_lines1 + 255) / 256), 1, B), 256, c_n1 * sizeof(float), st>>>(d);
+        if ((rc = check_launch("bfm_gen_finish"))) return rc;
+        k_gen_prefilter_z<<<dim3((unsigned)((c_rows2 + kCubicLines - 1) / kCubicLines), 1, B), 128, smem_z, st>>>(d);
+        if ((rc = check_launch("bfm_gen_finish"))) return rc;
+        k_gen_cubic_zoom<<<dim3((s1 + kUR - 1) / kUR, s0, B), threads, smem_c, st>>>(d, c_ny);
+        if ((rc = check_launch("bfm_gen_finish"))) return rc;
+    }
+    if (linear) {
+        if (smem > 40 * 1024)
+            cudaFuncSetAttribute(k_gen_upsample, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        k_gen_upsample<<<dim3((s1 + kUR - 1) / kUR, s0, B), threads, smem, st>>>(d, lz, ny);
+        rc = check_launch("bfm_gen_finish");
+        if (rc) return rc;
+    }
     if (vec) {
         k_gen_normalize<4><<<dim3((unsigned)((plane / 4 + 255) / 256), s0, B), 256, 0, st>>>(d);
         rc = check_launch("bfm_gen_finish");
@@ -1787,6 +2048,12 @@ int bfm_gen_finish(const bfm_gen_sample *h, const bfm_gen_sample *d, int B, void
         rc = check_launch("bfm_gen_finish");
     }
     return rc;
+}
+
+int bfm_gen_zoom_coords(int n_in, int n_out, float *out_dev, void *stream) {
+    if (n_in <= 0 || n_out <= 0 || !out_dev) return fail(BFM_E_INVALID, "%s", "bfm_gen_zoom_coords: bad argument");
+    k_gen_zoom_coords<<<(n_out + 255) / 256, 256, 0, (cudaStream_t)stream>>>(n_in, n_out, out_dev);
+    return check_launch("bfm_gen_zoom_coords");
 }
 
 int bfm_gen_run(const bfm_gen_sample *h, const bfm_gen_sample *d, int B, void *stream) {

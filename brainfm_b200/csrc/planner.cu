@@ -398,6 +398,7 @@ int plan_item(const bfm_plan_cfg &cfg, const bfm_plan_item &it, const bfm_plan_o
         s.seed = native ? splitmix64(seed ^ splitmix64(0x5eedull + sample0 + k)) : 0;
         // ---- buffers
         s.flip = st.flip;
+        s.zoom_order = cfg.bspline_zooming ? 3 : 0;          // draws nothing (datasets.py:337-340)
         if (!mode) { s.syn = o.syn; s.syn_pair_ok = (int)o.syn_pair_ok; }
         s.i_bf = o.i_bf; s.tmp[0] = o.tmp[0]; s.tmp[1] = o.tmp[1]; s.lowres = o.lowres;
         s.out = o.out; s.bflog_out = mode == 4 ? nullptr : o.bflog_out; s.residual = o.residual;

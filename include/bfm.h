@@ -267,6 +267,12 @@ typedef struct bfm_gen_sample {
        (k_gen_warp_pk: half the load requests of the two-volume gather, packed f32x2 arithmetic).  Results are
        identical to the unpaired path. */
     int syn_pair_ok;
+    /* Zoom back to the training grid (bfm_gen_finish; Generator/datasets.py:337-340).  0: myzoom_torch, the linear
+       zoom through `utab`.  3: the generator's `bspline_zooming`, i.e. interpol.resize(I, shape=size, anchor='edge',
+       interpolation=3, bound='dct2', prefilter=True): the dct2 cubic B-spline prefilter runs in place on `lowres`
+       (dead after the finish stage), then a cubic pull at the edge-anchored coordinates; `utab` is not read.  The
+       undegraded class keeps its direct path (see n_band).  Any other value: BFM_E_INVALID. */
+    int zoom_order;
     /* Slab mode, optional: 2 ints of device scratch.  With x_count > 0, bfm_gen_bbox also reduces the source x range
        [gmm_xr[0], gmm_xr[1]) that the OWNED output planes gather from (same clamped coordinates as the bounding box,
        floor(min) .. 1 + ceil(max)), and bfm_gen_gmm only synthesises those planes of the crop: the bounding box --
@@ -289,6 +295,10 @@ int bfm_gen_gmm(const bfm_gen_sample *s_host, const bfm_gen_sample *s_dev, int B
 int bfm_gen_warp(const bfm_gen_sample *s_host, const bfm_gen_sample *s_dev, int B, void *stream);
 int bfm_gen_resample(const bfm_gen_sample *s_host, const bfm_gen_sample *s_dev, int B, void *stream);
 int bfm_gen_finish(const bfm_gen_sample *s_host, const bfm_gen_sample *s_dev, int B, void *stream);
+/* Test hook, not part of the generator API: the sample coordinates of the cubic zoom back (zoom_order 3) along one
+ * axis, n_in -> n_out: out_dev[o] = o * (n_in/n_out) + 0.5 * (n_in/n_out - 1), evaluated on the device in float32 by
+ * the same device function bfm_gen_finish uses, so that the parity tests can pin them bit for bit. */
+int bfm_gen_zoom_coords(int n_in, int n_out, float *out_dev, void *stream);
 /* all six stages back to back */
 int bfm_gen_run(const bfm_gen_sample *s_host, const bfm_gen_sample *s_dev, int B, void *stream);
 
@@ -332,6 +342,7 @@ typedef struct bfm_plan_cfg {
     double ct_prob, mix_synth_prob;
     int8_t ct_group[256];           /* -1, or 0..3 = darker, dark, bright, brighter (constants.py) */
     int n_samples;                  /* samples per item: 1 (BaseGen) or all_samples (BrainIDGen) */
+    int bspline_zooming;            /* != 0: every descriptor gets zoom_order = 3 (cubic zoom back); draws nothing */
     bfm_plan_aug aug[BFM_PLAN_MAX_SAMPLES];        /* synthetic inputs (generator + [mild|severe] + synth_image_generator) */
     bfm_plan_aug aug_real[BFM_PLAN_MAX_SAMPLES];   /* real-image inputs (... + real_image_generator) */
     /* directories indexed by n_in = 0..size[a]: fwd = zoom by size/n_in (small grids -> training grid),
