@@ -357,7 +357,7 @@ class NativePlanner:
     # ---- one batch ---------------------------------------------------------------------------------------
     def run(self, indices, timers=None, patch=None, plan_only=False):
         """Plan the batch in the library and run the fused chain.
-        patch(descs, info): optional hook called after planning and BEFORE the descriptors travel to the device (slab
+        patch(descs): optional hook called after planning and BEFORE the descriptors travel to the device (slab
         mode sets x_begin / x_count there, which depend on the planned flip).  plan_only: stop after the upload and
         return the plan (descs, device address, info, output tensors) without launching any stage."""
         ds, L = self.ds, _lib.lib()
@@ -453,7 +453,7 @@ class NativePlanner:
         arena.used = used.value
         st = _stream()
         if patch is not None:
-            patch(descs, info)
+            patch(descs)
             C.memmove(slot["host"].data_ptr() + (descs_dev.value - slot["dev"].data_ptr()), C.addressof(descs),
                       C.sizeof(descs))
         nbytes = (upload.value + 15) // 16 * 16

@@ -181,6 +181,17 @@ def test_slab_mode_without_injected_draws_does_not_depend_on_the_decomposition(w
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-3000:]
 
 
+@pytest.mark.parametrize("planner", ["python", "native"])
+def test_slab_mode_refuses_a_rank_without_planes(planner):
+    """More ranks than planes: a rank that owns no plane raises instead of generating a slab.  Of 2 s0 + 1 ranks the
+    middle one owns no plane whether the volume is flipped (slabs mirrored) or not."""
+    from brainfm_b200.Generator.slab import generate_slab
+    _, ds, _ = cuda_case("g64_s0", None, planner=planner, run=lambda d: None)
+    s0 = int(ds.size[0])
+    with pytest.raises(ValueError, match="owns no plane"):
+        generate_slab(ds, 0, rank=s0, world=2 * s0 + 1)
+
+
 @pytest.mark.parametrize("name", ["g64_s0", "g64_s2", "g160_s0"])
 def test_full_bbox_scan_equals_candidate_result(name):
     """bfm_gen_bbox: with the candidate lists disabled (ncand = 0) the persistent full scan must give the same six
