@@ -23,7 +23,7 @@ from ..draws import HostDraws
 from ..plan import Arena, band_host, device_tables, set_zoom_tab, zoom_newsize
 from . import constants as K
 from .utils import (DeformDict, DeformPlan, _stream, fast_3D_interp_torch, make_affine_matrix, myzoom_torch,
-                    read_and_deform_image, resolution_sampler, scratch_stride)
+                    read_and_deform_image, read_and_deform_segmentation, resolution_sampler, scratch_stride)
 
 ct_brightness_group = {
     'darker': [4, 5, 14, 15, 24, 31, 72],
@@ -163,6 +163,7 @@ class BaseGen(Dataset):
         nlat = int((n_labels - nn_) / 2.0)
         self.vflip = np.concatenate([np.array(range(nn_)), np.array(range(nn_ + nlat, n_labels)),
                                      np.array(range(nn_, nn_ + nlat))])
+        self._vflip32 = np.ascontiguousarray(self.vflip, dtype=np.int32)      # bfm_gen_segmentation's vflip_host
 
     def get_info(self, t1):
         hit = self._info.get(t1)
@@ -629,6 +630,12 @@ class BaseGen(Dataset):
         stage('bbox', L.bfm_gen_bbox, d_dev)
         for job in jobs:
             job['plan'].have_bbox = True
+        seg = [(b, job['seg_cls']) for b, job in enumerate(jobs) if job.get('seg_cls') is not None]
+        if seg:
+            seg_all = self._segmentation_stage(descs, d_dev, B, seg, timers=timers)
+            self._keep.append(seg_all)
+            for q, (b, _) in enumerate(seg):
+                jobs[b]['seg_out'] = seg_all[q]
         if targets_fn is not None:
             if timers is not None:
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -876,11 +883,56 @@ class BaseGen(Dataset):
                 target[key] = fused['aux_out'][key]          # written by the fused chain (warp + finish stages)
             else:
                 target.update(self.read_and_deform_target(idx, target.keys(), key, input_mode, setups, deform_dict))
+        seg = ctx.get('seg_job')
         for task_name in self.tasks:
-            if task_name in K.processing_funcs.keys() and task_name not in ['T1', 'T2', 'FLAIR']:
+            if task_name == 'segmentation' and seg is not None:
+                target[task_name] = seg['seg_out']               # written by bfm_gen_segmentation
+            elif task_name in K.processing_funcs.keys() and task_name not in ['T1', 'T2', 'FLAIR']:
                 target.update(self.read_and_deform_target(idx, target.keys(), task_name, input_mode, setups,
                                                           deform_dict))
         return target
+
+    # ---- segmentation target of the fused chain (bfm_gen_segmentation) ------------------------------------------
+    def _seg_stage_ok(self):
+        """The segmentation target can come from the batched stage: it is asked for, the stock reader is registered
+        (a replaced reader keeps running op-wise) and the one-hots are hard ones over both hemispheres."""
+        a = self.synth_args
+        return ('segmentation' in self.tasks and not a.deform_one_hots and not a.left_hemis_only and
+                K.processing_funcs.get('segmentation') is read_and_deform_segmentation)
+
+    def _seg_classes(self, path, src):
+        """uint8 class map lut[S] (labels < 0 or >= len(lut) -> 0, as read_and_deform_segmentation) of the segmentation
+        volume at `path`, built once and kept in the volume cache beside it (an upload / refresh of the volume drops
+        it); None when the volume does not have the label map's shape `src`."""
+        S = self.cache.get(path, 'i32')
+        if list(S.shape) != [int(v) for v in src]:
+            return None
+
+        def build():
+            n = self.lut.numel()
+            cls = self.lut[S.clamp(0, n - 1).long()]
+            return torch.where((S >= 0) & (S < n), cls, torch.zeros_like(cls)).to(torch.uint8).contiguous()
+        return self.cache.derived('seg_classes', (path,), build)
+
+    def _segmentation_stage(self, descs, d_dev, n_desc, pairs, out=None, timers=None):
+        """bfm_gen_segmentation over [(descriptor index, class map)], one job per item, after bfm_gen_bbox: the
+        (len(pairs), n_classes, *size) one-hot targets, written into `out` when given."""
+        n_cls, N = int(self.onehotmatrix.shape[0]), int(np.prod(self.size))
+        if out is None:
+            out = torch.empty((len(pairs), n_cls, *self.size), dtype=torch.float32, device=self.device)
+        jobs = (_lib.GenSeg * len(pairs))()
+        base = out.data_ptr()
+        for q, (b, cls) in enumerate(pairs):
+            jobs[q].sample, jobs[q].cls, jobs[q].out = b, cls.data_ptr(), base + 4 * q * n_cls * N
+        if timers is not None:
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            e0.record()
+        _lib.check(_lib.lib().bfm_gen_segmentation(C.addressof(descs), d_dev, n_desc, jobs, len(pairs), n_cls,
+                                                   self._vflip32.ctypes.data, _stream()))
+        if timers is not None:
+            e1.record()
+            timers.setdefault('segmentation', []).append((e0, e1))
+        return out
 
     def _fused_image_targets(self, ctx, jobs):
         """Real-image targets (T1/T2/FLAIR, read_and_deform_image) that can ride on the synthetic image's gather:
@@ -961,6 +1013,7 @@ class BaseGen(Dataset):
             return native.run(indices, timers=timers)
         arena = self.arena.begin()
         ctxs, jobs, spans, slow = [], [], [], {}
+        seg_ok = self._seg_stage_ok()
         for n, idx in enumerate(indices):
             ctx = self._prologue_host(idx, arena)
             ctxs.append(ctx)
@@ -983,6 +1036,11 @@ class BaseGen(Dataset):
             if aux:
                 jobs[first]['aux'] = aux
                 ctx['fused_job'] = jobs[first]
+            if seg_ok:                                   # one segmentation per item, on its first descriptor
+                cls = self._seg_classes(ctx['modalities']['segmentation'], ctx['deform']['_plan'].src)
+                if cls is not None:
+                    jobs[first]['seg_cls'] = cls
+                    ctx['seg_job'] = jobs[first]
 
         def run_targets():
             for n, ctx in enumerate(ctxs):

@@ -42,7 +42,6 @@ class NativePlanner:
         self._prep_version = -1
         self._items = {}
         self._item_version = -1
-        self._other_targets = None
 
     _KEYS = ('photo_prob', 'pathology_prob', 'random_shape_prob', 'flip_prob', 'max_rotation', 'max_shear',
              'max_scaling', 'nonlin_scale_min', 'nonlin_scale_max', 'nonlin_std_max', 'ct_prob', 'low_res_only',
@@ -219,16 +218,28 @@ class NativePlanner:
 
     # ---- one batch, lean path ------------------------------------------------------------------------------
     def fast_ok(self):
-        """run_fast covers native draws with every requested target riding on the fused gather (no op-wise target
-        readers, no replay, no stage timers)."""
+        """run_fast covers native draws with every requested target riding on the fused gather or coming from the
+        batched segmentation stage (no op-wise target readers, no replay, no stage timers).  `bias_field` and `CT`
+        targets are the 0. placeholder of a subject without that file (per item, see `_item_entry`)."""
         ds = self.ds
         if getattr(ds.rng, 'replay', False):
             return False
-        other = self._other_targets
-        if other is None:
-            other = self._other_targets = any(t in K.processing_funcs and t not in ('T1', 'T2', 'FLAIR')
-                                              for t in ds.tasks)
-        return not other
+        for t in ds.tasks:
+            if t not in K.processing_funcs or t in ('T1', 'T2', 'FLAIR', 'CT', 'bias_field'):
+                continue
+            if t == 'segmentation' and ds._seg_stage_ok():
+                continue
+            return False
+        return True
+
+    def _seg_item(self, mods, src):
+        """The segmentation path when the item's segmentation target comes from the batched stage, else None (op-wise
+        reader)."""
+        ds = self.ds
+        if not ds._seg_stage_ok():
+            return None
+        path = mods['segmentation']
+        return None if ds._seg_classes(path, src) is None else path
 
     def _item_entry(self, idx):
         """Per-INDEX cached PlanItem bytes + metadata (valid while the device cache holds the same tensors)."""
@@ -241,8 +252,13 @@ class NativePlanner:
             return ent
         prep = self._prepare([idx], use_cache=False)
         meta = prep['metas'][0]
+        mods = meta[4]
+        # the class map itself is looked up per batch: the cache drops it when the segmentation is uploaded
+        seg = self._seg_item(mods, meta[6]) if 'segmentation' in ds.tasks else None
+        ok = self.item_ok(ds.idx_to_path(idx)[1], mods) and ('segmentation' not in ds.tasks or seg is not None) and \
+            not any(t in mods for t in ('CT', 'bias_field') if t in ds.tasks)
         ent = dict(raw=bytes(prep['items']), meta=meta, keys=prep['keys'], n_aux=len(meta[5]),
-                   src_pad=prep['src_pad'], ok=self.item_ok(ds.idx_to_path(idx)[1], meta[4]),
+                   src_pad=prep['src_pad'], ok=ok, seg=seg,
                    needs_plan=len(meta[5]) < sum(1 for k in ('T1', 'T2', 'FLAIR') if k in meta[4]),
                    case_name=_case_name(meta[2]))
         if self._item_version != cache.version:              # volumes were loaded while preparing
@@ -305,6 +321,9 @@ class NativePlanner:
         bfl = torch.empty((total, 1, *size), dtype=torch.float32, device=dev) if want_bflog else None
         res = torch.empty((total, 1, *size), dtype=torch.float32, device=dev) if want_res else None
         aux_all = torch.empty((n_aux_total, 1, *size), dtype=torch.float32, device=dev) if n_aux_total else None
+        n_seg = sum(1 for e in ents if e['seg'] is not None)
+        seg = torch.empty((n_seg, int(ds.onehotmatrix.shape[0]), *size), dtype=torch.float32, device=dev) \
+            if n_seg else None
         if als is not None:
             torch.cuda.set_stream(lane_stream)
         if tr is not None:
@@ -345,14 +364,18 @@ class NativePlanner:
             tr.append(('plan_run', _t.perf_counter()))
         self.counter += B
         arena.used = arena.committed = used.value
+        cls = None
+        if seg is not None:                    # reads the descriptors and boxes of this arena slot: before mark_done
+            cls = [(n * ns, ds._seg_classes(e['seg'], e['meta'][6])) for n, e in enumerate(ents) if e['seg'] is not None]
+            ds._segmentation_stage(descs, descs_dev.value, total, cls, out=seg)
         arena.mark_done()
         self.last = dict(descs=descs, descs_dev=descs_dev.value, info=info, total=total,
-                         keep=(out, bfl, res, aux_all, items), arena_slot=arena.cur)
+                         keep=(out, bfl, res, aux_all, items, seg, cls), arena_slot=arena.cur)
         if tr is not None:
             tr.append(('done', _t.perf_counter()))
         ds._last_descs = (descs, descs_dev.value, total)
         ds._last_out = out
-        return LazyItems(ds, ents, info, ns, out, bfl, res, aux_all)
+        return LazyItems(ds, ents, info, ns, out, bfl, res, aux_all, seg)
 
     # ---- one batch ---------------------------------------------------------------------------------------
     def run(self, indices, timers=None, patch=None, plan_only=False):
@@ -467,10 +490,12 @@ class NativePlanner:
                         arena=arena, metas=metas)
         # ---- per-item context (targets that do not ride on the fused gather need a DeformPlan)
         h, d_dev = C.addressof(descs), descs_dev.value
-        other_targets = self._other_targets
-        if other_targets is None:
-            other_targets = self._other_targets = any(t in K.processing_funcs and t not in ('T1', 'T2', 'FLAIR')
-                                                      for t in ds.tasks)
+        # segmentation targets of the batched stage (bfm_gen_segmentation); every other target task is op-wise
+        seg_ok = ds._seg_stage_ok()
+        seg_cls = [ds._seg_classes(m[4]['segmentation'], m[6]) if seg_ok else None for m in metas]
+        other_targets = any(t in K.processing_funcs and t not in ('T1', 'T2', 'FLAIR', 'segmentation') for t in ds.tasks)
+        if 'segmentation' in ds.tasks and any(c is None for c in seg_cls):
+            other_targets = True
         need_plans = other_targets or any(len(m[5]) < sum(1 for k in ('T1', 'T2', 'FLAIR') if k in m[4]) for m in metas)
 
         def setups_of(inf):
@@ -501,6 +526,13 @@ class NativePlanner:
         else:
             stage('plan', L.bfm_gen_plan)
             stage('bbox', L.bfm_gen_bbox)
+        seg_views = [None] * B
+        seg_jobs = [(n * ns, c) for n, c in enumerate(seg_cls) if c is not None]
+        if seg_jobs:
+            seg_all = ds._segmentation_stage(descs, d_dev, total, seg_jobs, timers=timers)
+            keep += [seg_all, seg_cls]
+            it = iter(seg_all.unbind(0))
+            seg_views = [next(it) if c is not None else None for c in seg_cls]
         aux_views = aux_all.unbind(0) if aux_all is not None else ()
         k_aux = 0
         targets = []
@@ -523,11 +555,12 @@ class NativePlanner:
                                                             ctx['setups'], deform))
                 else:
                     target[key] = 0.
-            if other_targets:
-                for task_name in ds.tasks:
-                    if task_name in K.processing_funcs.keys() and task_name not in ('T1', 'T2', 'FLAIR'):
-                        target.update(ds.read_and_deform_target(ctx['idx'], target.keys(), task_name,
-                                                                ctx['input_mode'], ctx['setups'], deform))
+            for task_name in ds.tasks:
+                if task_name == 'segmentation' and seg_views[n] is not None:
+                    target[task_name] = seg_views[n]
+                elif task_name in K.processing_funcs.keys() and task_name not in ('T1', 'T2', 'FLAIR'):
+                    target.update(ds.read_and_deform_target(ctx['idx'], target.keys(), task_name,
+                                                            ctx['input_mode'], ctx['setups'], deform))
             target['pathology'] = 0.
             target['pathology_prob'] = 0.
             targets.append(target)
@@ -621,21 +654,26 @@ class LazyItems:
     `(datasets_num, dataset_name, input_mode, target, sample)` -- a sequence: len(), indexing and iteration build
     them exactly as `NativePlanner.run` does."""
 
-    def __init__(self, ds, ents, info, ns, out, bfl, res, aux_all):
+    def __init__(self, ds, ents, info, ns, out, bfl, res, aux_all, seg=None):
         self._ds, self._ents, self._info, self._ns = ds, ents, info, ns
         self.input, self.bias_field_log, self.high_res_residual = out, bfl, res
         self._aux = aux_all
+        self._seg = seg
         self._built = None
 
     @property
     def targets(self):
-        """{key: (n_items_with_that_target, 1, *size)} of the fused real-image targets, in item order."""
+        """{key: (n_items_with_that_target, 1, *size)} of the fused real-image targets, in item order, and
+        'segmentation': the (B, n_classes, *size) one-hots when the task is on."""
         out, k = {}, 0
         for e in self._ents:
             for key, _ in e['meta'][5]:
                 out.setdefault(key, []).append(self._aux[k])
                 k += 1
-        return {key: torch.stack(v) for key, v in out.items()}
+        out = {key: torch.stack(v) for key, v in out.items()}
+        if self._seg is not None:
+            out['segmentation'] = self._seg
+        return out
 
     def _build(self):
         if self._built is not None:
@@ -645,6 +683,8 @@ class LazyItems:
         bfl_v = self.bias_field_log.unbind(0) if self.bias_field_log is not None else None
         res_v = self.high_res_residual.unbind(0) if self.high_res_residual is not None else None
         aux_v = self._aux.unbind(0) if self._aux is not None else ()
+        seg_v = self._seg.unbind(0) if self._seg is not None else None
+        others = [t for t in ds.tasks if t in K.processing_funcs and t not in ('T1', 'T2', 'FLAIR')]
         tuples, k_aux = [], 0
         for n, e in enumerate(self._ents):
             idx, dataset_name, t1_path, age, mods, aux, src = e['meta']
@@ -657,6 +697,8 @@ class LazyItems:
                 k_aux += 1
             for key in ('T1', 'T2', 'FLAIR'):
                 target[key] = fused[key] if key in fused else 0.
+            for key in others:              # segmentation, or the 0. of a file the subject does not have (fast_ok)
+                target[key] = seg_v[n] if key == 'segmentation' else 0.
             target['pathology'] = 0.
             target['pathology_prob'] = 0.
             if age is not None:

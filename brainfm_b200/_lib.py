@@ -50,6 +50,10 @@ class GenSample(C.Structure):
                 ("zoom_order", c_i), ("gmm_xr", c_p)]
 
 
+class GenSeg(C.Structure):
+    _fields_ = [("sample", c_i), ("cls", c_p), ("out", c_p)]
+
+
 # ---- native host planner (bfm_plan_batch) ----------------------------------------------------------------
 PLAN_MAX_SAMPLES = 16
 c_d = C.c_double
@@ -134,6 +138,7 @@ _PROTOS = {
     "bfm_gen_finish": (c_i, [c_p, c_p, c_i, c_p]),
     "bfm_gen_zoom_coords": (c_i, [c_i, c_i, c_p, c_p]),
     "bfm_gen_run": (c_i, [c_p, c_p, c_i, c_p]),
+    "bfm_gen_segmentation": (c_i, [c_p, c_p, c_i, c_p, c_i, c_i, c_p, c_p]),
     "bfm_plan_batch": (c_i, [c_p, c_i, c_p, c_p, c_u64, c_u64, c_p, c_p, c_i64, C.POINTER(c_i64), C.POINTER(c_i64),
                              c_p, C.POINTER(c_p), c_p, c_p, c_i64, C.POINTER(c_i64)]),
     "bfm_plan_run": (c_i, [c_p, c_i, c_p, c_p, c_u64, c_u64, c_p, c_p, c_i64, c_i64, C.POINTER(c_i64), c_p,

@@ -1654,6 +1654,79 @@ __global__ void __launch_bounds__(256) k_gen_normalize(const bfm_gen_sample *__r
     }
 }
 
+// ---------------------------------------------------------------------------------------------- segmentation
+// The one-hot target is (n_classes x 4) bytes per voxel written and ~1 byte read: the stage is bound by HBM writes.
+// A warp first gathers the class of each voxel of its rows (deform_rows, k_label_warp's rounding and clamping) into
+// shared memory, then writes the rows channel by channel, each lane owning 4 consecutive z voxels per 128-bit
+// streaming store (evict-first, so that the one-hot does not push the other pipeline lane's volumes out of L2).
+// When size[2] % 4 != 0 the rows do not start on 16-byte boundaries and every store is scalar.
+constexpr int kSegMaxJobs = 64, kSegMaxClasses = 64;
+struct SegParams {
+    int n_classes;
+    int vflip[kSegMaxClasses];
+    bfm_gen_seg jobs[kSegMaxJobs];
+};
+
+template <bool VEC>
+__global__ void __launch_bounds__(kRowWarps * 32)
+k_gen_segmentation(const bfm_gen_sample *__restrict__ S, const __grid_constant__ SegParams P, int fstride, int cstride) {
+    extern __shared__ float smem[];
+    __shared__ bfm_gen_sample sd;
+    const bfm_gen_seg &job = P.jobs[blockIdx.z];
+    stage_desc(&sd, S + job.sample);
+    const bfm_deform &d = sd.d;
+    const DefRegs g = load_def(d);
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    float *smF = smem + warp * kRowsPerWarp * fstride;
+    uint8_t *smC = (uint8_t *)(smem + kRowWarps * kRowsPerWarp * fstride) + warp * kRowsPerWarp * cstride;
+    const int n_rows = g.s0 * g.s1;
+    const int row0 = (blockIdx.x * kRowWarps + warp) * kRowsPerWarp;
+    if (row0 >= n_rows) return;
+    const int *bb = sd.bbox;
+    const int n1 = d.src[1], n2 = d.src[2];
+    const int b0 = bb[0], b1 = bb[1], b2 = bb[2];
+    const int cx = bb[3] - b0, cy = bb[4] - b1, cz = bb[5] - b2;
+    const float l0 = (float)b0, l1 = (float)b1, l2 = (float)b2;
+    const uint8_t *__restrict__ cls = job.cls;
+    deform_rows<kRowsPerWarp>(
+        d, g, smF, row0, n_rows, lane, [](int) {},
+        [&](int r, int, int, int, int k, float px, float py, float pz) {
+            const int x = min(max(__float2int_rn(__fsub_rn(px, l0)), 0), cx - 1) + b0;
+            const int y = min(max(__float2int_rn(__fsub_rn(py, l1)), 0), cy - 1) + b1;
+            const int z = min(max(__float2int_rn(__fsub_rn(pz, l2)), 0), cz - 1) + b2;
+            smC[r * cstride + k] = __ldg(cls + (x * n1 + y) * n2 + z);
+        });
+    __syncwarp();
+    const int nr = min(kRowsPerWarp, n_rows - row0);
+    const int64_t N = (int64_t)n_rows * g.s2;
+    const bool flip = sd.flip != 0;
+    const int nc = P.n_classes;
+    float *__restrict__ out = job.out;
+    if (VEC) {
+        const int G = g.s2 >> 2;
+        const int64_t N4 = N >> 2;
+        for (int q = lane; q < nr * G; q += 32) {
+            const int r = q / G, k4 = (q - r * G) << 2;
+            const int row = row0 + r, i = row / g.s1, j = row - i * g.s1;
+            const uchar4 c4 = *(const uchar4 *)(smC + r * cstride + k4);
+            float4 *o = (float4 *)(out + ((int64_t)((flip ? g.s0 - 1 - i : i) * g.s1 + j) * g.s2 + k4));
+            for (int c = 0; c < nc; ++c) {
+                const int sc = flip ? P.vflip[c] : c;
+                __stcs(o + c * N4, make_float4(c4.x == sc ? 1.f : 0.f, c4.y == sc ? 1.f : 0.f, c4.z == sc ? 1.f : 0.f,
+                                               c4.w == sc ? 1.f : 0.f));
+            }
+        }
+    } else {
+        for (int q = lane; q < nr * g.s2; q += 32) {
+            const int r = q / g.s2, k = q - r * g.s2;
+            const int row = row0 + r, i = row / g.s1, j = row - i * g.s1;
+            const int v = smC[r * cstride + k];
+            float *o = out + ((int64_t)((flip ? g.s0 - 1 - i : i) * g.s1 + j) * g.s2 + k);
+            for (int c = 0; c < nc; ++c) __stcs(o + c * N, v == (flip ? P.vflip[c] : c) ? 1.f : 0.f);
+        }
+    }
+}
+
 static inline bool misaligned(const void *p, uintptr_t bytes) { return ((uintptr_t)p & (bytes - 1)) != 0; }
 
 static int check_batch(const bfm_gen_sample *h, const bfm_gen_sample *d, int B) {
@@ -2064,6 +2137,64 @@ int bfm_gen_run(const bfm_gen_sample *h, const bfm_gen_sample *d, int B, void *s
     if ((rc = bfm_gen_warp(h, d, B, stream))) return rc;
     if ((rc = bfm_gen_resample(h, d, B, stream))) return rc;
     return bfm_gen_finish(h, d, B, stream);
+}
+
+int bfm_gen_segmentation(const bfm_gen_sample *h, const bfm_gen_sample *d, int n_desc, const bfm_gen_seg *jobs,
+                         int n_jobs, int n_classes, const int32_t *vflip, void *stream) {
+    if (!h || !d || n_desc <= 0 || !jobs || n_jobs <= 0 || !vflip)
+        return fail(BFM_E_INVALID, "%s", "bfm_gen_segmentation: null descriptors, jobs or vflip, or nothing to do");
+    if (n_classes < 1 || n_classes > kSegMaxClasses)
+        return fail(BFM_E_INVALID, "%s", "bfm_gen_segmentation: n_classes must be 1..64");
+    SegParams P;
+    P.n_classes = n_classes;
+    for (int c = 0; c < n_classes; ++c) {
+        if (vflip[c] < 0 || vflip[c] >= n_classes)
+            return fail(BFM_E_INVALID, "%s", "bfm_gen_segmentation: vflip entry outside [0, n_classes)");
+        P.vflip[c] = vflip[c];
+    }
+    const int *size = nullptr;
+    int fstride = 0;
+    for (int q = 0; q < n_jobs; ++q) {
+        const bfm_gen_seg &jb = jobs[q];
+        if (jb.sample < 0 || jb.sample >= n_desc)
+            return fail(BFM_E_INVALID, "%s", "bfm_gen_segmentation: job sample outside the descriptor array");
+        if (!jb.cls || !jb.out) return fail(BFM_E_INVALID, "%s", "bfm_gen_segmentation: null class map or output");
+        if (misaligned(jb.out, 16)) return fail(BFM_E_INVALID, "%s", "bfm_gen_segmentation: output not 16-byte aligned");
+        const bfm_gen_sample &s = h[jb.sample];
+        if (!s.bbox) return fail(BFM_E_INVALID, "%s", "bfm_gen_segmentation: descriptor without bounding box");
+        for (int a = 0; a < 3; ++a)
+            if (s.d.size[a] <= 0 || s.d.src[a] <= 0)
+                return fail(BFM_E_INVALID, "%s", "bfm_gen_segmentation: non-positive size");
+        if ((int64_t)s.d.src[0] * s.d.src[1] * s.d.src[2] >= (1LL << 31) ||
+            (int64_t)s.d.size[0] * s.d.size[1] * s.d.size[2] >= (1LL << 31))
+            return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen_segmentation: volumes of 2^31 voxels or more are not supported");
+        if (s.d.fsmall && !s.d.F_full && (s.d.fs[2] > kMaxSmallZ || s.d.fs[2] <= 0))
+            return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen_segmentation: deformation small grid too deep");
+        if (size && (s.d.size[0] != size[0] || s.d.size[1] != size[1] || s.d.size[2] != size[2]))
+            return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen_segmentation: all jobs share the output size");
+        size = s.d.size;
+        if (s.d.fsmall && !s.d.F_full) fstride = max(fstride, s.d.fs[2] * 3);
+    }
+    const int cstride = (size[2] + 3) & ~3;
+    const size_t smem = (size_t)kRowWarps * kRowsPerWarp * (fstride * sizeof(float) + cstride);
+    if (smem > 200 * 1024) return fail(BFM_E_UNSUPPORTED, "%s", "bfm_gen_segmentation: rows too long for shared memory");
+    const bool vec = (size[2] & 3) == 0;
+    if (smem > 40 * 1024)
+        cudaFuncSetAttribute(vec ? (const void *)k_gen_segmentation<true> : (const void *)k_gen_segmentation<false>,
+                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const int64_t rows = (int64_t)size[0] * size[1];
+    const int per_block = kRowWarps * kRowsPerWarp;
+    const dim3 grid((unsigned)((rows + per_block - 1) / per_block), 1, 1);
+    cudaStream_t st = (cudaStream_t)stream;
+    for (int base = 0; base < n_jobs; base += kSegMaxJobs) {
+        const int nb = min(kSegMaxJobs, n_jobs - base);
+        for (int q = 0; q < nb; ++q) P.jobs[q] = jobs[base + q];
+        if (vec) k_gen_segmentation<true><<<dim3(grid.x, 1, nb), kRowWarps * 32, smem, st>>>(d, P, fstride, cstride);
+        else k_gen_segmentation<false><<<dim3(grid.x, 1, nb), kRowWarps * 32, smem, st>>>(d, P, fstride, cstride);
+        int rc = check_launch("bfm_gen_segmentation");
+        if (rc) return rc;
+    }
+    return BFM_OK;
 }
 
 }  // extern "C"

@@ -302,6 +302,22 @@ int bfm_gen_zoom_coords(int n_in, int n_out, float *out_dev, void *stream);
 /* all six stages back to back */
 int bfm_gen_run(const bfm_gen_sample *s_host, const bfm_gen_sample *s_dev, int B, void *stream);
 
+/* Segmentation target of the fused chain (read_and_deform_segmentation, Generator/utils.py:394-424, with
+ * deform_one_hots off): one job per ITEM, all jobs in one launch.  A job warps its class map through the deformation,
+ * bounding box and flip of descriptor s_dev[sample] (nearest, round-half-even, clamped to the crop: the arithmetic of
+ * bfm_label_warp_onehot) and writes the (n_classes, size) float32 one-hot, flipped along axis 0 with output channel c
+ * holding input channel vflip_host[c] when the descriptor's flip is set.  Must run after bfm_gen_bbox and before the
+ * descriptors' arena slot is reused.
+ *   cls: the class map of the item's segmentation, lut applied (labels < 0 or >= lut_n -> 0), uint8, source shape;
+ *   out: 16-byte aligned.  n_classes 1..64, vflip_host[c] in [0, n_classes); all jobs share the output size. */
+typedef struct bfm_gen_seg {
+    int sample;             /* index into the descriptor array */
+    const uint8_t *cls;
+    float *out;
+} bfm_gen_seg;
+int bfm_gen_segmentation(const bfm_gen_sample *s_host, const bfm_gen_sample *s_dev, int n_desc, const bfm_gen_seg *jobs,
+                         int n_jobs, int n_classes, const int32_t *vflip_host, void *stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Native host planner: every per-sample scalar draw and all the scalar set-up arithmetic of
  * BaseGen.__getitem__ / BrainIDGen.__getitem__ for synthetic inputs with the stock augmentation chain, in the
