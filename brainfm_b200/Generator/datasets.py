@@ -20,10 +20,11 @@ from torch.utils.data import Dataset
 
 from .. import _lib, io as bio
 from ..draws import HostDraws
-from ..plan import Arena, band_host, device_tables, set_zoom_tab, zoom_newsize
+from ..plan import Arena, band_host, device_tables
 from . import constants as K
 from .utils import (DeformDict, DeformPlan, _stream, fast_3D_interp_torch, make_affine_matrix, myzoom_torch,
-                    read_and_deform_image, read_and_deform_segmentation, resolution_sampler, scratch_stride)
+                    read_and_deform_image, read_and_deform_segmentation, resolution_sampler, scratch_stride,
+                    syn_stride)
 
 ct_brightness_group = {
     'darker': [4, 5, 14, 15, 24, 31, 72],
@@ -465,6 +466,24 @@ class BaseGen(Dataset):
             self._ws[name] = t
         return t
 
+    def _scratch(self, n_samples, n_aux, stride):
+        """Base addresses of the fused chain's per-sample scratch for n_samples samples and n_aux fused real-image
+        targets: syn (`stride` floats per sample), i_bf, tmp (two slots per sample), lowres and aux_raw (one slot per
+        target; 0 without targets), slots of scratch_stride(N) floats."""
+        syn = self._workspace('syn', n_samples * stride, zero=True)
+        # syn is zero-initialised once and afterwards only ever holds finite values; when its stride changes the slots
+        # move and stale data no longer lines up: start clean
+        if self._ws.get('syn_stride') != stride:
+            if 'syn_stride' in self._ws:
+                syn.zero_()
+            self._ws['syn_stride'] = stride
+        s0, s1, s2 = self.size
+        Np = scratch_stride(s0 * s1 * s2)
+        return (syn.data_ptr(), self._workspace('i_bf', n_samples * Np).data_ptr(),
+                self._workspace('tmp', n_samples * 2 * Np).data_ptr(),
+                self._workspace('lowres', n_samples * Np).data_ptr(),
+                self._workspace('aux_raw', n_aux * Np).data_ptr() if n_aux else 0)
+
     def _build_descs(self, jobs, arena):
         """Fill one bfm_gen_sample per job.  Per sample only the small random grids and the two 256-entry
         tables travel through the arena; zoom tables come from the device-resident cache, the banded
@@ -481,21 +500,9 @@ class BaseGen(Dataset):
         bfl_all = torch.empty((n_bfl, 1, *size), dtype=torch.float32, device=dev) if n_bfl else None
         res_all = torch.empty((n_res, 1, *size), dtype=torch.float32, device=dev) if n_res else None
         aux_all = torch.empty((n_aux, 1, *size), dtype=torch.float32, device=dev) if n_aux else None
-        # persistent scratch: syn is zero-initialised once and afterwards only ever holds finite values
-        src_pad = max(int(np.prod(j['plan'].src)) + j['plan'].src[1] * j['plan'].src[2] + j['plan'].src[2] + 1
-                      for j in jobs)
-        src_pad = 2 * ((src_pad + 3) // 4 * 4)         # room for float2 {synthetic, T1} pairs (syn_pair_ok)
-        syn_ws = self._workspace('syn', B * src_pad, zero=True)
-        if self._ws.get('syn_stride') != src_pad:      # slots moved: stale data no longer lines up, start clean
-            if 'syn_stride' in self._ws:
-                syn_ws.zero_()
-            self._ws['syn_stride'] = src_pad
+        stride = max(syn_stride(j['plan'].src) for j in jobs)
+        p_syn, p_ibf, p_tmp, p_low, p_raw = self._scratch(B, n_aux, stride)
         Np = scratch_stride(N)
-        i_bf_ws = self._workspace('i_bf', B * Np)
-        tmp_ws = self._workspace('tmp', B * 2 * Np)
-        low_ws = self._workspace('lowres', B * Np)
-        raw_ws = self._workspace('aux_raw', n_aux * Np) if n_aux else None
-        p_syn, p_ibf, p_tmp, p_low = syn_ws.data_ptr(), i_bf_ws.data_ptr(), tmp_ws.data_ptr(), low_ws.data_ptr()
         keep = [out, bfl_all, res_all, aux_all]
         results = []
         k_bfl = k_res = k_aux = 0
@@ -519,7 +526,7 @@ class BaseGen(Dataset):
                     e = p['eps_gmm'].to(dev).contiguous()
                     keep.append(e)
                     s.eps_gmm = e.data_ptr()
-                s.syn = p_syn + 4 * b * src_pad
+                s.syn = p_syn + 4 * b * stride
                 s.syn_pair_ok = 1 if self.pair_mode else 0
             s.seed = int(p['seed'])
             s.bbox = plan.bbox_ptr
@@ -593,7 +600,7 @@ class BaseGen(Dataset):
                 s.aux_mm, _ = arena.reserve(8 * _lib.MAX_AUX)
             for c, (key, vol) in enumerate(aux):
                 s.aux_src[c] = vol.data_ptr()
-                s.aux_raw[c] = raw_ws.data_ptr() + 4 * k_aux * Np
+                s.aux_raw[c] = p_raw + 4 * k_aux * Np
                 s.aux_out[c] = aux_all[k_aux].data_ptr()
                 job['aux_out'][key] = aux_all[k_aux]
                 k_aux += 1
@@ -952,8 +959,9 @@ class BaseGen(Dataset):
                 out.append((key, vol))
         return out[:_lib.MAX_AUX]
 
-    def _native_planner(self, indices):
-        """The NativePlanner to use for this batch, or None (Python planner)."""
+    def _native_planner(self, indices=None, strict=True):
+        """The NativePlanner to use for this batch, or None (Python planner); indices=None checks the configuration
+        only.  With planner='native' a batch the library cannot plan raises, unless strict=False."""
         if self.planner == 'python':
             return None
         from .native import NativePlanner
@@ -963,8 +971,8 @@ class BaseGen(Dataset):
                 self._native = NativePlanner(self)
             else:
                 self._native.refresh()
-            ok = self._native.batch_ok(indices)
-        if not ok and self.planner == 'native':
+            ok = indices is None or self._native.batch_ok(indices)
+        if not ok and strict and self.planner == 'native':
             raise NotImplementedError("this configuration needs the Python planner (planner='python' or 'auto')")
         return self._native if ok else None
 
@@ -1068,16 +1076,8 @@ class BaseGen(Dataset):
         if self.planner == 'python':
             return None
         self.cache.begin_batch()
-        from .native import NativePlanner
-        if not (NativePlanner.config_ok(self) and (self.planner == 'native' or type(self.rng) is HostDraws)):
-            return None
-        if self._native is None:
-            self._native = NativePlanner(self)
-        else:
-            self._native.refresh()
-        if not self._native.fast_ok():
-            return None
-        return self._native.run_fast(indices)
+        native = self._native_planner(strict=False)          # run_fast checks the batch's items itself
+        return native.run_fast(indices) if native is not None and native.fast_ok() else None
 
     def _slow_item(self, ctx):
         """Op-by-op path: real-image inputs, custom augmentation sequences, pathology."""

@@ -10,15 +10,16 @@ random grids drawn on the device.
 With a `ReplayDraws` source the planner runs in replay mode and consumes the recorded draws (parity tests).
 """
 import ctypes as C
+import os
+import time
 from collections import defaultdict
 
 import numpy as np
 import torch
 
 from .. import _lib
-from ..draws import HostDraws
 from . import constants as K
-from .utils import DeformDict, DeformPlan, _stream, scratch_stride
+from .utils import DeformDict, DeformPlan, _stream, syn_stride
 
 
 def _ptr(t):
@@ -38,10 +39,8 @@ class NativePlanner:
         self.cfg = self._build_cfg()
         self._fp = self.fingerprint()
         self.last = None
-        self._prep = {}
-        self._prep_version = -1
-        self._items = {}
-        self._item_version = -1
+        self._ents = {}                  # dataset index -> _entry
+        self._version = -1               # cache.version the entries were built under
 
     _KEYS = ('photo_prob', 'pathology_prob', 'random_shape_prob', 'flip_prob', 'max_rotation', 'max_shear',
              'max_scaling', 'nonlin_scale_min', 'nonlin_scale_max', 'nonlin_std_max', 'ct_prob', 'low_res_only',
@@ -151,76 +150,127 @@ class NativePlanner:
         self._keep += [dirs, ident]
         return cfg
 
-    # ---- per-batch preparation, cached ------------------------------------------------------------------
-    def _prepare(self, indices, use_cache=True):
-        """PlanItem array + per-item metadata of a batch of dataset indices.  Everything in here depends only on the
-        indices and on WHICH tensors the device cache holds, so it is built once per index tuple and reused until the
-        cache's membership changes (`DeviceVolumeCache.version`: a new volume, an eviction, a clear); uploads and
-        refreshes overwrite cached volumes in place and keep it valid.  On a hit the volumes are only touched (LRU
-        order + eviction epoch).  Saves ~0.15 ms of ctypes stores and dictionary look-ups per batch of 8."""
-        ds = self.ds
-        key = tuple(int(i) for i in indices)
-        cache = ds.cache
-        if self._prep_version != cache.version:
-            self._prep.clear()               # entries hold references to cached tensors: drop them with the old set
-            self._prep_version = cache.version
-        ent = self._prep.get(key)
-        if use_cache and ent is not None and ent['version'] == cache.version:
+    # ---- per-index preparation, cached ---------------------------------------------------------------------
+    def _entry(self, idx):
+        """PlanItem bytes + metadata of one dataset index.  Everything in here depends only on the index and on WHICH
+        tensors the device cache holds, so it is built once per index and reused until the cache's membership changes
+        (`DeviceVolumeCache.version`: a new volume, an eviction, a clear); uploads and refreshes overwrite cached
+        volumes in place and keep it valid.  On a hit the volumes are touched (LRU order + eviction epoch), so that
+        looking up the batch's other entries cannot evict them.  What depends on the task list is decided per batch."""
+        ds, cache = self.ds, self.ds.cache
+        if self._version != cache.version:
+            self._ents.clear()               # entries point at cached tensors: drop them with the old set
+            self._version = cache.version
+        ent = self._ents.get(idx)
+        if ent is not None:
             cache.touch(ent['keys'])
             return ent
-        B = len(key)
-        items = (_lib.PlanItem * B)()
-        metas, keys = [], []
-        n_aux_total, src_pad = 0, 0
-        for n, idx in enumerate(key):
-            dataset_name, input_prob, t1_path, age = ds.idx_to_path(idx)
-            mods = ds.get_info(t1_path)
-            lab = cache.get(mods['Gen'], 'gen')
-            keys.append((mods['Gen'], 'gen'))
-            it = items[n]
-            it.labels = lab.data_ptr()
-            it.label_is_u8 = 1 if lab.dtype == torch.uint8 else 0
-            src = [int(v) for v in lab.shape[:3]]
-            it.src[:] = src
-            for q, m in enumerate(('T1', 'T2', 'FLAIR', 'CT')):
-                it.input_prob[q] = float(input_prob.get(m, 0))
-            for q, m in enumerate(('T1', 'T2', 'FLAIR')):
-                if m in mods and input_prob.get(m, 0) > 0:
-                    it.real_vol[q] = cache.get(mods[m], 'f32').data_ptr()
-                    keys.append((mods[m], 'f32'))
-            if 'CT' in mods and input_prob.get('CT', 0) > 0:
-                it.ct_vol = cache.get(mods['CT'], 'f32').data_ptr()
-                keys.append((mods['CT'], 'f32'))
-            aux = ds._fused_aux_volumes(mods, src)
-            it.n_aux = len(aux)
-            for c, (k_, vol) in enumerate(aux):
-                it.aux_src[c] = vol.data_ptr()
-                keys.append((mods[k_], 'f32'))
-            n_aux_total += len(aux)
-            src_pad = max(src_pad, src[0] * src[1] * src[2] + src[1] * src[2] + src[2] + 1)
-            metas.append((idx, dataset_name, t1_path, age, dict(mods), aux, src))
-        ent = dict(items=items, metas=metas, n_aux_total=n_aux_total, src_pad=src_pad, keys=keys,
-                   version=cache.version, ok=None)
-        if use_cache:
-            if len(self._prep) > 256 or self._prep_version != cache.version:      # volumes were loaded while preparing
-                self._prep.clear()
-                self._prep_version = cache.version
-            self._prep[key] = ent
+        dataset_name, input_prob, t1_path, age = ds.idx_to_path(idx)
+        mods = dict(ds.get_info(t1_path))
+        lab = cache.get(mods['Gen'], 'gen')
+        keys = [(mods['Gen'], 'gen')]
+        it = _lib.PlanItem()
+        it.labels = lab.data_ptr()
+        it.label_is_u8 = 1 if lab.dtype == torch.uint8 else 0
+        src = [int(v) for v in lab.shape[:3]]
+        it.src[:] = src
+        for q, m in enumerate(('T1', 'T2', 'FLAIR', 'CT')):
+            it.input_prob[q] = float(input_prob.get(m, 0))
+        for q, m in enumerate(('T1', 'T2', 'FLAIR')):
+            if m in mods and input_prob.get(m, 0) > 0:
+                it.real_vol[q] = cache.get(mods[m], 'f32').data_ptr()
+                keys.append((mods[m], 'f32'))
+        if 'CT' in mods and input_prob.get('CT', 0) > 0:
+            it.ct_vol = cache.get(mods['CT'], 'f32').data_ptr()
+            keys.append((mods['CT'], 'f32'))
+        aux = ds._fused_aux_volumes(mods, src)
+        it.n_aux = len(aux)
+        for c, (k, vol) in enumerate(aux):
+            it.aux_src[c] = vol.data_ptr()
+            keys.append((mods[k], 'f32'))
+        ent = dict(raw=bytes(it), keys=keys, idx=idx, dataset_name=dataset_name, case_name=_case_name(t1_path),
+                   age=age, mods=mods, src=src, aux=[k for k, _ in aux], syn_stride=syn_stride(src),
+                   item_ok=self.item_ok(input_prob, mods),
+                   # every real-image target the subject has rides on the gather (else: op-wise readers, run)
+                   all_fused=len(aux) == sum(1 for k in ('T1', 'T2', 'FLAIR') if k in mods))
+        if self._version != cache.version:              # volumes were loaded while preparing
+            self._ents.clear()
+            self._version = cache.version
+        self._ents[idx] = ent
         return ent
 
     def batch_ok(self, indices):
-        """item_ok for every index of the batch (cached with the batch's preparation)."""
+        """item_ok for every index of the batch."""
+        return all(self._entry(int(i))['item_ok'] for i in indices)
+
+    @staticmethod
+    def _items(ents):
+        """A fresh PlanItem array of the batch (the layout writes the target pointers into it, replay the injected
+        draws), its number of fused real-image targets and its syn stride."""
+        items = (_lib.PlanItem * len(ents))()
+        isz, base = C.sizeof(_lib.PlanItem), C.addressof(items)
+        n_aux, stride = 0, 0
+        for n, e in enumerate(ents):
+            C.memmove(base + n * isz, e['raw'], isz)
+            n_aux += len(e['aux'])
+            if e['syn_stride'] > stride:
+                stride = e['syn_stride']
+        return items, n_aux, stride
+
+    def _seg_maps(self, ents):
+        """Per item: the class map of the batched segmentation stage (bfm_gen_segmentation), or None (no segmentation
+        target, or the op-wise reader).  Looked up per batch: the cache drops a map when its volume is uploaded."""
         ds = self.ds
-        ent = self._prepare(indices)
-        if ent['ok'] is None:
-            ent['ok'] = all(self.item_ok(ds.idx_to_path(m[0])[1], m[4]) for m in ent['metas'])
-        return ent['ok']
+        if not ds._seg_stage_ok():
+            return [None] * len(ents)
+        return [ds._seg_classes(e['mods']['segmentation'], e['src']) for e in ents]
+
+    def _outputs(self, total, n_aux, n_seg):
+        """(out, bias_field_log, high_res_residual, fused targets, segmentation) tensors of a batch.  They come from
+        the CALLER's stream pool when a pipeline set one (DevicePipeline): the caching allocator keeps one pool of free
+        blocks per stream, and with the outputs in the lanes' pools a lane was measured to run out of free 131 MB blocks
+        and cudaMalloc three new ones (1.3-200 ms) while a dozen sat free in the other pools.  Safe: every submit()
+        orders the lane after the caller's stream, so a block the consumer freed is only rewritten after the consumer's
+        work on it (see pipeline._DeviceTicket.wait)."""
+        ds, size, dev = self.ds, self.size, self.device
+        als = getattr(ds, '_alloc_stream', None)
+        if als is not None:
+            lane_stream = torch.cuda.current_stream(dev)
+            torch.cuda.set_stream(als)
+        shape = (total, 1, *size)
+        out = torch.empty(shape, dtype=torch.float32, device=dev)
+        bfl = torch.empty(shape, dtype=torch.float32, device=dev) if ds._want_bflog('synth') else None
+        res = torch.empty(shape, dtype=torch.float32, device=dev) if 'super_resolution' in ds.tasks else None
+        aux = torch.empty((n_aux, 1, *size), dtype=torch.float32, device=dev) if n_aux else None
+        seg = torch.empty((n_seg, int(ds.onehotmatrix.shape[0]), *size), dtype=torch.float32, device=dev) \
+            if n_seg else None
+        if als is not None:
+            torch.cuda.set_stream(lane_stream)
+        return out, bfl, res, aux, seg
+
+    def _bufs(self, outputs, n_aux, stride):
+        """bfm_step_bufs of a batch: base addresses of its outputs and of the persistent scratch (BaseGen._scratch)."""
+        out, bfl, res, aux, _ = outputs
+        bufs = _lib.StepBufs()
+        bufs.out, bufs.bflog_out, bufs.residual, bufs.aux_out = _ptr(out), _ptr(bfl), _ptr(res), _ptr(aux)
+        bufs.syn, bufs.i_bf, bufs.tmp, bufs.lowres, bufs.aux_raw = self.ds._scratch(out.shape[0], n_aux, stride)
+        bufs.syn_stride = stride
+        bufs.pair_ok = 1 if self.ds.pair_mode else 0
+        return bufs
+
+    def _keep_last(self, descs, d_dev, info, arena, outputs, *keep):
+        """The last batch's plan (tests, bench.py's `last_shapes`) and what its kernels still read or write."""
+        total = len(descs)
+        self.last = dict(descs=descs, descs_dev=d_dev, info=info, total=total, keep=(outputs,) + keep,
+                         arena_slot=arena.cur)
+        self.ds._last_descs = (descs, d_dev, total)
+        self.ds._last_out = outputs[0]
 
     # ---- one batch, lean path ------------------------------------------------------------------------------
     def fast_ok(self):
         """run_fast covers native draws with every requested target riding on the fused gather or coming from the
         batched segmentation stage (no op-wise target readers, no replay, no stage timers).  `bias_field` and `CT`
-        targets are the 0. placeholder of a subject without that file (per item, see `_item_entry`)."""
+        targets are the 0. placeholder of a subject without that file (checked per item by run_fast)."""
         ds = self.ds
         if getattr(ds.rng, 'replay', False):
             return False
@@ -232,41 +282,6 @@ class NativePlanner:
             return False
         return True
 
-    def _seg_item(self, mods, src):
-        """The segmentation path when the item's segmentation target comes from the batched stage, else None (op-wise
-        reader)."""
-        ds = self.ds
-        if not ds._seg_stage_ok():
-            return None
-        path = mods['segmentation']
-        return None if ds._seg_classes(path, src) is None else path
-
-    def _item_entry(self, idx):
-        """Per-INDEX cached PlanItem bytes + metadata (valid while the device cache holds the same tensors)."""
-        ds, cache = self.ds, self.ds.cache
-        if self._item_version != cache.version:
-            self._items.clear()
-            self._item_version = cache.version
-        ent = self._items.get(idx)
-        if ent is not None:
-            return ent
-        prep = self._prepare([idx], use_cache=False)
-        meta = prep['metas'][0]
-        mods = meta[4]
-        # the class map itself is looked up per batch: the cache drops it when the segmentation is uploaded
-        seg = self._seg_item(mods, meta[6]) if 'segmentation' in ds.tasks else None
-        ok = self.item_ok(ds.idx_to_path(idx)[1], mods) and ('segmentation' not in ds.tasks or seg is not None) and \
-            not any(t in mods for t in ('CT', 'bias_field') if t in ds.tasks)
-        ent = dict(raw=bytes(prep['items']), meta=meta, keys=prep['keys'], n_aux=len(meta[5]),
-                   src_pad=prep['src_pad'], ok=ok, seg=seg,
-                   needs_plan=len(meta[5]) < sum(1 for k in ('T1', 'T2', 'FLAIR') if k in meta[4]),
-                   case_name=_case_name(meta[2]))
-        if self._item_version != cache.version:              # volumes were loaded while preparing
-            self._items.clear()
-            self._item_version = cache.version
-        self._items[idx] = ent
-        return ent
-
     def run_fast(self, indices):
         """generate_batch for the common case in ONE library call (bfm_plan_run: buffer lay-out, planning, descriptor
         upload, every stage launch) and a few dozen microseconds of Python: per-index cached PlanItems are copied into
@@ -276,106 +291,56 @@ class NativePlanner:
         ds, L = self.ds, _lib.lib()
         tr = getattr(ds, '_trace', None)           # development aid: host time stamps of the last call
         if tr is not None:
-            import time as _t
             tr.clear()
-            tr.append(('start', _t.perf_counter()))
-        B = len(indices)
-        ns = self.n_samples
-        total = B * ns
+            tr.append(('start', time.perf_counter()))
+        absent = [t for t in ('CT', 'bias_field') if t in ds.tasks]      # only as the 0. of a file the item lacks
         ents = []
-        for idx in indices:
-            e = self._item_entry(int(idx))
-            if not e['ok'] or e['needs_plan']:
+        for i in indices:
+            e = self._entry(int(i))
+            if not (e['item_ok'] and e['all_fused']) or absent and not e['mods'].keys().isdisjoint(absent):
                 return None
             ents.append(e)
+        B, ns = len(ents), self.n_samples
+        total = B * ns
+        cls = self._seg_maps(ents)
+        jobs = [(n * ns, c) for n, c in enumerate(cls) if c is not None]
+        if 'segmentation' in ds.tasks and len(jobs) < B:
+            return None
         if self.seed is None:
             self.seed = int(np.random.randint(0, 2 ** 62))
         ds.hemis_mask = None
-        size, N, dev = self.size, self.N, self.device
-        items = (_lib.PlanItem * B)()
-        isz = C.sizeof(_lib.PlanItem)
-        base = C.addressof(items)
-        touch = ds.cache.touch
-        n_aux_total, src_pad = 0, 0
-        for n, e in enumerate(ents):
-            C.memmove(base + n * isz, e['raw'], isz)
-            touch(e['keys'])
-            n_aux_total += e['n_aux']
-            if e['src_pad'] > src_pad:
-                src_pad = e['src_pad']
-        src_pad = (src_pad + 3) // 4 * 4 * 2                 # float2 {synthetic, target} pairs (syn_pair_ok)
+        items, n_aux, stride = self._items(ents)
         if tr is not None:
-            tr.append(('items', _t.perf_counter()))
-        want_bflog = ds._want_bflog('synth')
-        want_res = 'super_resolution' in ds.tasks
-        # Outputs come from the CALLER's stream pool when a pipeline set one (DevicePipeline): the caching allocator keeps
-        # one pool of free blocks per stream, and with the outputs in the lanes' pools a lane was measured to run out of
-        # free 131 MB blocks and cudaMalloc three new ones (1.3-200 ms) while a dozen sat free in the other pools.  Safe:
-        # every submit() orders the lane after the caller's stream, so a block the consumer freed is only rewritten
-        # after the consumer's work on it (see pipeline._DeviceTicket.wait).
-        als = getattr(ds, '_alloc_stream', None)
-        if als is not None:
-            lane_stream = torch.cuda.current_stream(dev)
-            torch.cuda.set_stream(als)
-        out = torch.empty((total, 1, *size), dtype=torch.float32, device=dev)
-        bfl = torch.empty((total, 1, *size), dtype=torch.float32, device=dev) if want_bflog else None
-        res = torch.empty((total, 1, *size), dtype=torch.float32, device=dev) if want_res else None
-        aux_all = torch.empty((n_aux_total, 1, *size), dtype=torch.float32, device=dev) if n_aux_total else None
-        n_seg = sum(1 for e in ents if e['seg'] is not None)
-        seg = torch.empty((n_seg, int(ds.onehotmatrix.shape[0]), *size), dtype=torch.float32, device=dev) \
-            if n_seg else None
-        if als is not None:
-            torch.cuda.set_stream(lane_stream)
+            tr.append(('items', time.perf_counter()))
+        outputs = self._outputs(total, n_aux, len(jobs))
         if tr is not None:
-            tr.append(('outputs', _t.perf_counter()))
-        syn_ws = ds._workspace('syn', total * src_pad, zero=True)
-        if ds._ws.get('syn_stride') != src_pad:
-            if 'syn_stride' in ds._ws:
-                syn_ws.zero_()
-            ds._ws['syn_stride'] = src_pad
-        bufs = _lib.StepBufs()
-        bufs.out = out.data_ptr()
-        bufs.bflog_out = bfl.data_ptr() if bfl is not None else None
-        bufs.residual = res.data_ptr() if res is not None else None
-        bufs.syn = syn_ws.data_ptr()
-        bufs.syn_stride = src_pad
-        Np = scratch_stride(N)
-        bufs.i_bf = ds._workspace('i_bf', total * Np).data_ptr()
-        bufs.tmp = ds._workspace('tmp', total * 2 * Np).data_ptr()
-        bufs.lowres = ds._workspace('lowres', total * Np).data_ptr()
-        if n_aux_total:
-            bufs.aux_out = aux_all.data_ptr()
-            bufs.aux_raw = ds._workspace('aux_raw', n_aux_total * Np).data_ptr()
-        bufs.pair_ok = 1 if ds.pair_mode else 0
+            tr.append(('outputs', time.perf_counter()))
+        bufs = self._bufs(outputs, n_aux, stride)
         if tr is not None:
-            tr.append(('workspaces', _t.perf_counter()))
+            tr.append(('workspaces', time.perf_counter()))
         arena = ds.arena.begin()
         if tr is not None:
-            tr.append(('arena', _t.perf_counter()))
+            tr.append(('arena', time.perf_counter()))
         slot = arena.slots[arena.cur]
         descs = (_lib.GenSample * total)()
         descs_dev = C.c_void_p(0)
         info = (_lib.PlanInfo * B)()
         used = C.c_int64(0)
-        _lib.check(L.bfm_plan_run(C.addressof(self.cfg), B, base, C.addressof(bufs), self.seed, self.counter,
-                                  slot["host"].data_ptr(), slot["dev"].data_ptr(), arena.capacity, arena.used,
-                                  C.byref(used), C.addressof(descs), C.byref(descs_dev), C.addressof(info), _stream()))
+        _lib.check(L.bfm_plan_run(C.addressof(self.cfg), B, C.addressof(items), C.addressof(bufs), self.seed,
+                                  self.counter, slot["host"].data_ptr(), slot["dev"].data_ptr(), arena.capacity,
+                                  arena.used, C.byref(used), C.addressof(descs), C.byref(descs_dev), C.addressof(info),
+                                  _stream()))
         if tr is not None:
-            tr.append(('plan_run', _t.perf_counter()))
+            tr.append(('plan_run', time.perf_counter()))
         self.counter += B
         arena.used = arena.committed = used.value
-        cls = None
-        if seg is not None:                    # reads the descriptors and boxes of this arena slot: before mark_done
-            cls = [(n * ns, ds._seg_classes(e['seg'], e['meta'][6])) for n, e in enumerate(ents) if e['seg'] is not None]
-            ds._segmentation_stage(descs, descs_dev.value, total, cls, out=seg)
+        if jobs:                               # reads the descriptors and boxes of this arena slot: before mark_done
+            ds._segmentation_stage(descs, descs_dev.value, total, jobs, out=outputs[4])
         arena.mark_done()
-        self.last = dict(descs=descs, descs_dev=descs_dev.value, info=info, total=total,
-                         keep=(out, bfl, res, aux_all, items, seg, cls), arena_slot=arena.cur)
+        self._keep_last(descs, descs_dev.value, info, arena, outputs, items, cls)
         if tr is not None:
-            tr.append(('done', _t.perf_counter()))
-        ds._last_descs = (descs, descs_dev.value, total)
-        ds._last_out = out
-        return LazyItems(ds, ents, info, ns, out, bfl, res, aux_all, seg)
+            tr.append(('done', time.perf_counter()))
+        return LazyItems(ds, ents, info, ns, outputs, cls)
 
     # ---- one batch ---------------------------------------------------------------------------------------
     def run(self, indices, timers=None, patch=None, plan_only=False):
@@ -384,8 +349,7 @@ class NativePlanner:
         mode sets x_begin / x_count there, which depend on the planned flip).  plan_only: stop after the upload and
         return the plan (descs, device address, info, output tensors) without launching any stage."""
         ds, L = self.ds, _lib.lib()
-        size, N, ns = self.size, self.N, self.n_samples
-        B = len(indices)
+        ns, B = self.n_samples, len(indices)
         total = B * ns
         dev = self.device
         rng = ds.rng
@@ -393,49 +357,15 @@ class NativePlanner:
         if self.seed is None and not replay:
             self.seed = int(np.random.randint(0, 2 ** 62))
         ds.hemis_mask = None
-        want_bflog = ds._want_bflog('synth')
-        want_res = 'super_resolution' in ds.tasks
-        # ---- items: volumes from the device cache (prepared once per index tuple, see _prepare)
-        prep = self._prepare(indices, use_cache=not replay)     # replayed draws park eps pointers in the items
-        items, metas, n_aux_total, src_pad = prep['items'], prep['metas'], prep['n_aux_total'], prep['src_pad']
-        src_pad = (src_pad + 3) // 4 * 4
-        # ---- outputs (fresh) and persistent scratch
-        out = torch.empty((total, 1, *size), dtype=torch.float32, device=dev)
-        bfl = torch.empty((total, 1, *size), dtype=torch.float32, device=dev) if want_bflog else None
-        res = torch.empty((total, 1, *size), dtype=torch.float32, device=dev) if want_res else None
-        aux_all = torch.empty((n_aux_total, 1, *size), dtype=torch.float32, device=dev) if n_aux_total else None
-        # syn holds float2 {synthetic, T1} pairs for samples with one fused target (bfm_gen_sample.syn_pair_ok)
-        src_pad *= 2
-        syn_ws = ds._workspace('syn', total * src_pad, zero=True)
-        if ds._ws.get('syn_stride') != src_pad:
-            if 'syn_stride' in ds._ws:
-                syn_ws.zero_()
-            ds._ws['syn_stride'] = src_pad
-        Np = scratch_stride(N)
-        p_ibf = ds._workspace('i_bf', total * Np).data_ptr()
-        p_tmp = ds._workspace('tmp', total * 2 * Np).data_ptr()
-        p_low = ds._workspace('lowres', total * Np).data_ptr()
-        p_raw = ds._workspace('aux_raw', n_aux_total * Np).data_ptr() if n_aux_total else 0
+        ents = [self._entry(int(i)) for i in indices]
+        items, n_aux, stride = self._items(ents)
+        cls = [None] * B if plan_only else self._seg_maps(ents)
+        jobs = [(n * ns, c) for n, c in enumerate(cls) if c is not None]
+        outputs = self._outputs(total, n_aux, len(jobs))
+        bufs = self._bufs(outputs, n_aux, stride)
         outs = (_lib.PlanOut * total)()
-        o_np = np.frombuffer(outs, dtype=np.uint64).reshape(total, 9)
-        q = np.arange(total, dtype=np.uint64)
-        step, pstep = np.uint64(4 * N), np.uint64(4 * Np)
-        o_np[:, 0] = np.uint64(out.data_ptr()) + q * step
-        o_np[:, 1] = (np.uint64(bfl.data_ptr()) + q * step) if want_bflog else 0
-        o_np[:, 2] = (np.uint64(res.data_ptr()) + q * step) if want_res else 0
-        o_np[:, 3] = np.uint64(syn_ws.data_ptr()) + q * np.uint64(4 * src_pad)
-        o_np[:, 4] = np.uint64(p_ibf) + q * pstep
-        o_np[:, 5] = np.uint64(p_tmp) + (2 * q) * pstep
-        o_np[:, 6] = np.uint64(p_tmp) + (2 * q + 1) * pstep
-        o_np[:, 7] = np.uint64(p_low) + q * pstep
-        o_np[:, 8] = 1 if ds.pair_mode else 0
-        k_aux = 0
-        for n in range(B):
-            it = items[n]
-            for c in range(it.n_aux):
-                it.aux_out[c] = aux_all.data_ptr() + 4 * N * k_aux
-                it.aux_raw[c] = p_raw + 4 * Np * k_aux
-                k_aux += 1
+        _lib.check(L.bfm_plan_layout(C.addressof(self.cfg), B, C.addressof(items), C.addressof(bufs),
+                                     C.addressof(outs)))
         # ---- draws to replay (parity tests): scalars and small arrays flattened in log order
         keep = []
         flat, n_flat = None, 0
@@ -482,35 +412,24 @@ class NativePlanner:
         nbytes = (upload.value + 15) // 16 * 16
         _lib.check(L.bfm_upload_pinned(slot["dev"].data_ptr() + start, slot["host"].data_ptr() + start, nbytes, st))
         arena.committed = arena.used
-        if plan_only:
-            self.last = dict(descs=descs, descs_dev=descs_dev.value, info=info, total=total,
-                             keep=(out, bfl, res, aux_all, keep), arena_slot=arena.cur)
-            ds._last_descs = (descs, descs_dev.value, total)
-            return dict(descs=descs, d_dev=descs_dev.value, info=info, out=out, bfl=bfl, res=res, aux=aux_all,
-                        arena=arena, metas=metas)
-        # ---- per-item context (targets that do not ride on the fused gather need a DeformPlan)
         h, d_dev = C.addressof(descs), descs_dev.value
-        # segmentation targets of the batched stage (bfm_gen_segmentation); every other target task is op-wise
-        seg_ok = ds._seg_stage_ok()
-        seg_cls = [ds._seg_classes(m[4]['segmentation'], m[6]) if seg_ok else None for m in metas]
-        other_targets = any(t in K.processing_funcs and t not in ('T1', 'T2', 'FLAIR', 'segmentation') for t in ds.tasks)
-        if 'segmentation' in ds.tasks and any(c is None for c in seg_cls):
-            other_targets = True
-        need_plans = other_targets or any(len(m[5]) < sum(1 for k in ('T1', 'T2', 'FLAIR') if k in m[4]) for m in metas)
+        if plan_only:
+            self._keep_last(descs, d_dev, info, arena, outputs, keep)
+            out, bfl, res, aux, _ = outputs
+            return dict(descs=descs, d_dev=d_dev, info=info, out=out, bfl=bfl, res=res, aux=aux, arena=arena,
+                        ents=ents)
+        # ---- per-item context (targets that do not ride on the fused gather need a DeformPlan)
+        need_plans = any(t in K.processing_funcs and t not in ('T1', 'T2', 'FLAIR', 'segmentation') for t in ds.tasks) \
+            or ('segmentation' in ds.tasks and any(c is None for c in cls)) or not all(e['all_fused'] for e in ents)
+        # the set-up dictionary is only read by the op-wise target readers (and kept as ds.last_setups)
+        setups = [_setups(info[n]) if (need_plans or n == B - 1) else None for n in range(B)]
+        deforms = [self._deform_dict(e['src'], descs[n * ns], info[n], arena) if need_plans else None
+                   for n, e in enumerate(ents)]
 
-        def setups_of(inf):
-            return {'resolution': np.array(inf.resolution[:]), 'thickness': np.array(inf.thickness[:]),
-                    'photo_mode': bool(inf.photo_mode), 'pathol_mode': False, 'pathol_random_shape': False,
-                    'spac': inf.spac if inf.photo_mode else None, 'flip': bool(inf.flip), 'hemis': 'both'}
-
-        ctxs = []
-        for n, (idx, dataset_name, t1_path, age, mods, aux, src) in enumerate(metas):
-            inf = info[n]
-            # the set-up dictionary is only read by the op-wise target readers (and kept as ds.last_setups)
-            setups = setups_of(inf) if (need_plans or n == B - 1) else None
-            ctxs.append(dict(idx=idx, dataset_name=dataset_name, case_name=_case_name(t1_path),
-                             input_mode=_INPUT_MODES[inf.input_mode],
-                             age=age, setups=setups, modalities=mods, aux=aux, src=src, n=n))
+        def read(n, key, target):
+            ds.modalities = ents[n]['mods']
+            return ds.read_and_deform_target(ents[n]['idx'], target.keys(), key, _INPUT_MODES[info[n].input_mode],
+                                             setups[n], deforms[n])
 
         def stage(name, fn):
             if timers is not None:
@@ -526,84 +445,24 @@ class NativePlanner:
         else:
             stage('plan', L.bfm_gen_plan)
             stage('bbox', L.bfm_gen_bbox)
-        seg_views = [None] * B
-        seg_jobs = [(n * ns, c) for n, c in enumerate(seg_cls) if c is not None]
-        if seg_jobs:
-            seg_all = ds._segmentation_stage(descs, d_dev, total, seg_jobs, timers=timers)
-            keep += [seg_all, seg_cls]
-            it = iter(seg_all.unbind(0))
-            seg_views = [next(it) if c is not None else None for c in seg_cls]
-        aux_views = aux_all.unbind(0) if aux_all is not None else ()
-        k_aux = 0
-        targets = []
-        for ctx in ctxs:
-            n = ctx['n']
-            target = defaultdict(ds._default_target)
-            target['name'] = ctx['case_name']
-            fused = {}
-            for key, _ in ctx['aux']:
-                fused[key] = aux_views[k_aux]
-                k_aux += 1
-            deform = self._deform_dict(ctx, descs[n * ns], info[n], arena) if need_plans else None
-            ctx['deform'] = deform
-            ds.modalities = ctx['modalities']
-            for key in ('T1', 'T2', 'FLAIR'):
-                if key in fused:
-                    target[key] = fused[key]
-                elif key in ctx['modalities']:
-                    target.update(ds.read_and_deform_target(ctx['idx'], target.keys(), key, ctx['input_mode'],
-                                                            ctx['setups'], deform))
-                else:
-                    target[key] = 0.
-            for task_name in ds.tasks:
-                if task_name == 'segmentation' and seg_views[n] is not None:
-                    target[task_name] = seg_views[n]
-                elif task_name in K.processing_funcs.keys() and task_name not in ('T1', 'T2', 'FLAIR'):
-                    target.update(ds.read_and_deform_target(ctx['idx'], target.keys(), task_name,
-                                                            ctx['input_mode'], ctx['setups'], deform))
-            target['pathology'] = 0.
-            target['pathology_prob'] = 0.
-            targets.append(target)
+        if jobs:
+            ds._segmentation_stage(descs, d_dev, total, jobs, out=outputs[4], timers=timers)
+        tuples = list(LazyItems(ds, ents, info, ns, outputs, cls, read))      # op-wise readers: after the bbox stage
         if timers is not None or need_plans:
             stage('gmm', L.bfm_gen_gmm)
             stage('warp', L.bfm_gen_warp)
             stage('resample', L.bfm_gen_resample)
             stage('finish', L.bfm_gen_finish)
         arena.mark_done()
-        # ---- results
-        out_v = out.unbind(0)
-        bfl_v = bfl.unbind(0) if bfl is not None else None
-        res_v = res.unbind(0) if res is not None else None
-        results = []
-        for q_ in range(total):
-            s = {}
-            if res_v is not None:
-                s['high_res_residual'] = res_v[q_]
-            s['input'] = out_v[q_]
-            if bfl_v is not None and info[q_ // ns].input_mode != 4:      # no bias field on CT inputs
-                s['bias_field_log'] = bfl_v[q_]
-            results.append(s)
-        tuples = []
-        for ctx, target in zip(ctxs, targets):
-            n = ctx['n']
-            sample = results[n * ns:(n + 1) * ns] if ds._list_samples else results[n * ns]
-            if ctx['age'] is not None:
-                target['age'] = ctx['age']
-            tuples.append((ds.datasets_num, ctx['dataset_name'], ctx['input_mode'], target, sample))
-        if ctxs:
-            ds.last_setups, ds.last_deform = ctxs[-1]['setups'], ctxs[-1]['deform']
-        self.last = dict(descs=descs, descs_dev=d_dev, info=info, total=total, keep=(out, bfl, res, aux_all, keep),
-                         arena_slot=arena.cur)
-        ds._last_descs = (descs, d_dev, total)
-        ds._last_out = out
+        ds.last_setups, ds.last_deform = setups[-1], deforms[-1]
+        self._keep_last(descs, d_dev, info, arena, outputs, cls, keep)
         return tuples
 
-    def _deform_dict(self, ctx, desc, inf, arena):
+    def _deform_dict(self, src, desc, inf, arena):
         """A DeformDict around the planned deformation, for targets computed by the op-wise entry points."""
-        ds = self.ds
         plan = DeformPlan.__new__(DeformPlan)
         plan.size = list(self.size)
-        plan.src = list(ctx['src'])
+        plan.src = list(src)
         plan.device = self.device
         plan.A_host = np.array(inf.A[:], dtype=np.float32).reshape(3, 3)
         plan.c2_host = np.array(inf.c2[:], dtype=np.float32)
@@ -643,22 +502,33 @@ class NativePlanner:
 _INPUT_MODES = ('synth', 'T1', 'T2', 'FLAIR', 'CT')
 
 
+def _setups(inf):
+    """The set-up dictionary of a planned item (what get_setup_params returns)."""
+    return {'resolution': np.array(inf.resolution[:]), 'thickness': np.array(inf.thickness[:]),
+            'photo_mode': bool(inf.photo_mode), 'pathol_mode': False, 'pathol_random_shape': False,
+            'spac': inf.spac if inf.photo_mode else None, 'flip': bool(inf.flip), 'hemis': 'both'}
+
+
 def _case_name(t1_path):
-    import os
     return os.path.basename(t1_path).split('.T1w.nii')[0]
 
 
-class LazyItems:
-    """What `run_fast` returns: the batch as collated device tensors (`input`: (B * n_samples, 1, *size), `bias_field_log`,
-    `high_res_residual`, `targets[key]`: (B, 1, *size)) and, on demand, the reference-shaped per-item tuples
-    `(datasets_num, dataset_name, input_mode, target, sample)` -- a sequence: len(), indexing and iteration build
-    them exactly as `NativePlanner.run` does."""
+def _absent(n, key, target):
+    return {key: 0.}                  # read_and_deform_target of a file the subject does not have
 
-    def __init__(self, ds, ents, info, ns, out, bfl, res, aux_all, seg=None):
-        self._ds, self._ents, self._info, self._ns = ds, ents, info, ns
-        self.input, self.bias_field_log, self.high_res_residual = out, bfl, res
-        self._aux = aux_all
-        self._seg = seg
+
+class LazyItems:
+    """The batch as collated device tensors (`input`: (B * n_samples, 1, *size), `bias_field_log`, `high_res_residual`,
+    `targets[key]`: (B, 1, *size)) and, on demand, the reference-shaped per-item tuples
+    `(datasets_num, dataset_name, input_mode, target, sample)` -- a sequence: len(), indexing and iteration build
+    them.  `run_fast` returns it; `run` lists it, with `read(n, key, target)` computing the op-wise targets of item n
+    (by default every target that neither rides on the fused gather nor comes from the segmentation stage is the 0. of
+    a file the subject does not have)."""
+
+    def __init__(self, ds, ents, info, ns, outputs, seg_maps, read=_absent):
+        self._ds, self._ents, self._info, self._ns, self._read = ds, ents, info, ns, read
+        self.input, self.bias_field_log, self.high_res_residual, self._aux, self._seg = outputs
+        self._seg_maps = seg_maps
         self._built = None
 
     @property
@@ -667,7 +537,7 @@ class LazyItems:
         'segmentation': the (B, n_classes, *size) one-hots when the task is on."""
         out, k = {}, 0
         for e in self._ents:
-            for key, _ in e['meta'][5]:
+            for key in e['aux']:
                 out.setdefault(key, []).append(self._aux[k])
                 k += 1
         out = {key: torch.stack(v) for key, v in out.items()}
@@ -678,31 +548,34 @@ class LazyItems:
     def _build(self):
         if self._built is not None:
             return self._built
-        ds, ns, info = self._ds, self._ns, self._info
+        ds, ns, info, read = self._ds, self._ns, self._info, self._read
         out_v = self.input.unbind(0)
         bfl_v = self.bias_field_log.unbind(0) if self.bias_field_log is not None else None
         res_v = self.high_res_residual.unbind(0) if self.high_res_residual is not None else None
-        aux_v = self._aux.unbind(0) if self._aux is not None else ()
-        seg_v = self._seg.unbind(0) if self._seg is not None else None
-        others = [t for t in ds.tasks if t in K.processing_funcs and t not in ('T1', 'T2', 'FLAIR')]
-        tuples, k_aux = [], 0
+        aux_v = iter(self._aux.unbind(0) if self._aux is not None else ())
+        seg_v = iter(self._seg.unbind(0) if self._seg is not None else ())
+        tuples = []
         for n, e in enumerate(self._ents):
-            idx, dataset_name, t1_path, age, mods, aux, src = e['meta']
             inf = info[n]
             target = defaultdict(ds._default_target)
             target['name'] = e['case_name']
-            fused = {}
-            for key, _ in aux:
-                fused[key] = aux_v[k_aux]
-                k_aux += 1
+            fused = {key: next(aux_v) for key in e['aux']}
             for key in ('T1', 'T2', 'FLAIR'):
-                target[key] = fused[key] if key in fused else 0.
-            for key in others:              # segmentation, or the 0. of a file the subject does not have (fast_ok)
-                target[key] = seg_v[n] if key == 'segmentation' else 0.
+                if key in fused:
+                    target[key] = fused[key]
+                elif key in e['mods']:
+                    target.update(read(n, key, target))
+                else:
+                    target[key] = 0.
+            for key in ds.tasks:
+                if key == 'segmentation' and self._seg_maps[n] is not None:
+                    target[key] = next(seg_v)
+                elif key in K.processing_funcs and key not in ('T1', 'T2', 'FLAIR'):
+                    target.update(read(n, key, target))
             target['pathology'] = 0.
             target['pathology_prob'] = 0.
-            if age is not None:
-                target['age'] = age
+            if e['age'] is not None:
+                target['age'] = e['age']
             results = []
             for q in range(n * ns, (n + 1) * ns):
                 smp = {}
@@ -713,7 +586,7 @@ class LazyItems:
                     smp['bias_field_log'] = bfl_v[q]
                 results.append(smp)
             sample = results if ds._list_samples else results[0]
-            tuples.append((ds.datasets_num, dataset_name, _INPUT_MODES[inf.input_mode], target, sample))
+            tuples.append((ds.datasets_num, e['dataset_name'], _INPUT_MODES[inf.input_mode], target, sample))
         self._built = tuples
         return tuples
 

@@ -76,7 +76,7 @@ def _plan_native(native, idx, patch):
     plan = native.run([idx], patch=patch, plan_only=True)
     descs = plan['descs']
     bfl = plan['bfl'][0] if plan['bfl'] is not None else None
-    keys = [k for k, _ in plan['metas'][0][5]]
+    keys = plan['ents'][0]['aux']
     return descs, plan['d_dev'], plan['arena'], bfl, keys, None, bool(descs[0].flip)
 
 

@@ -26,6 +26,14 @@ def scratch_stride(N):
     return (int(N) + 3) // 4 * 4
 
 
+def syn_stride(src):
+    """Floats per sample slot of the fused chain's `syn` scratch for a label map of shape `src`: float2 {synthetic,
+    target} pairs (bfm_gen_sample.syn_pair_ok) over the source volume with the volume cache's padding
+    (DeviceVolumeCache._pad), the volume rounded up to a multiple of 4 floats."""
+    s0, s1, s2 = (int(v) for v in src[:3])
+    return 2 * ((s0 * s1 * s2 + s1 * s2 + s2 + 1 + 3) // 4 * 4)
+
+
 def _need_cuda(t, what):
     if not isinstance(t, torch.Tensor) or not t.is_cuda:
         raise _lib.BfmError("%s must be a CUDA tensor: brainfm_b200 has no CPU path" % what)

@@ -141,6 +141,7 @@ _PROTOS = {
     "bfm_gen_segmentation": (c_i, [c_p, c_p, c_i, c_p, c_i, c_i, c_p, c_p]),
     "bfm_plan_batch": (c_i, [c_p, c_i, c_p, c_p, c_u64, c_u64, c_p, c_p, c_i64, C.POINTER(c_i64), C.POINTER(c_i64),
                              c_p, C.POINTER(c_p), c_p, c_p, c_i64, C.POINTER(c_i64)]),
+    "bfm_plan_layout": (c_i, [c_p, c_i, c_p, c_p, c_p]),
     "bfm_plan_run": (c_i, [c_p, c_i, c_p, c_p, c_u64, c_u64, c_p, c_p, c_i64, c_i64, C.POINTER(c_i64), c_p,
                            C.POINTER(c_p), c_p, c_p]),
     "bfm_interpol": (c_i, [c_i, c_i, c_p, c_p, c_p, C.POINTER(c_i), C.POINTER(c_i), C.POINTER(c_i), c_i, c_i, c_i,

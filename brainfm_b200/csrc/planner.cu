@@ -486,22 +486,17 @@ extern "C" int bfm_plan_batch(const bfm_plan_cfg *cfg, int n_items, const bfm_pl
     return BFM_OK;
 }
 
-// One call per batch for the common case (native draws, every target fused): lays the per-sample buffers out from a
-// handful of base pointers, plans, ships the descriptors and launches the whole chain.  Python then only allocates
-// the output tensors and makes this call (brainfm_b200/Generator/native.py::run_fast) -- the per-sample pointer
-// arithmetic, three ctypes calls and ~20 kernel launches of bfm_gen_run happen here, without the interpreter lock.
-extern "C" int bfm_plan_run(const bfm_plan_cfg *cfg, int n_items, bfm_plan_item *items, const bfm_step_bufs *bufs,
-                            uint64_t seed, uint64_t counter, void *arena_host, void *arena_dev, int64_t arena_capacity,
-                            int64_t arena_used_in, int64_t *arena_used_out, bfm_gen_sample *descs_host,
-                            void **descs_dev, bfm_plan_info *info, void *stream) {
-    if (!cfg || !items || !bufs || !arena_used_out || n_items <= 0 || n_items > 4096)
-        return fail(BFM_E_INVALID, "%s", "bfm_plan_run: null argument or bad batch size");
+// The per-sample buffer layout of a batch (include/bfm.h, bfm_step_bufs): bfm_plan_run and the general batch path
+// (brainfm_b200/Generator/native.py::run, before bfm_plan_batch) both lay their buffers out here.
+extern "C" int bfm_plan_layout(const bfm_plan_cfg *cfg, int n_items, bfm_plan_item *items, const bfm_step_bufs *bufs,
+                               bfm_plan_out *outs) {
+    if (!cfg || !items || !bufs || !outs || n_items <= 0 || n_items > 4096)
+        return fail(BFM_E_INVALID, "%s", "bfm_plan_layout: null argument or bad batch size");
     if (!bufs->out || !bufs->syn || !bufs->i_bf || !bufs->tmp || !bufs->lowres)
-        return fail(BFM_E_INVALID, "%s", "bfm_plan_run: null buffer");
-    const int ns = cfg->n_samples, total = n_items * ns;
+        return fail(BFM_E_INVALID, "%s", "bfm_plan_layout: null buffer");
+    const int total = n_items * cfg->n_samples;
     const int64_t N = (int64_t)cfg->size[0] * cfg->size[1] * cfg->size[2];
     const int64_t Np = (N + 3) & ~(int64_t)3;        // scratch slots keep the 16-byte alignment of their base
-    std::vector<bfm_plan_out> outs((size_t)total);
     for (int q = 0; q < total; ++q) {
         bfm_plan_out &o = outs[q];
         o.out = bufs->out + q * N;
@@ -517,15 +512,33 @@ extern "C" int bfm_plan_run(const bfm_plan_cfg *cfg, int n_items, bfm_plan_item 
     int64_t k_aux = 0;
     for (int n = 0; n < n_items; ++n)
         for (int c = 0; c < items[n].n_aux && c < BFM_MAX_AUX; ++c) {
-            if (!bufs->aux_out || !bufs->aux_raw) return fail(BFM_E_INVALID, "%s", "bfm_plan_run: null target buffer");
+            if (!bufs->aux_out || !bufs->aux_raw)
+                return fail(BFM_E_INVALID, "%s", "bfm_plan_layout: null target buffer");
             items[n].aux_out[c] = bufs->aux_out + k_aux * N;
             items[n].aux_raw[c] = bufs->aux_raw + k_aux * Np;
             ++k_aux;
         }
+    return BFM_OK;
+}
+
+// One call per batch for the common case (native draws, every target fused): lays the per-sample buffers out from a
+// handful of base pointers, plans, ships the descriptors and launches the whole chain.  Python then only allocates
+// the output tensors and makes this call (brainfm_b200/Generator/native.py::run_fast) -- the per-sample pointer
+// arithmetic, three ctypes calls and ~20 kernel launches of bfm_gen_run happen here, without the interpreter lock.
+extern "C" int bfm_plan_run(const bfm_plan_cfg *cfg, int n_items, bfm_plan_item *items, const bfm_step_bufs *bufs,
+                            uint64_t seed, uint64_t counter, void *arena_host, void *arena_dev, int64_t arena_capacity,
+                            int64_t arena_used_in, int64_t *arena_used_out, bfm_gen_sample *descs_host,
+                            void **descs_dev, bfm_plan_info *info, void *stream) {
+    if (!cfg || !items || !bufs || !arena_used_out || n_items <= 0 || n_items > 4096)
+        return fail(BFM_E_INVALID, "%s", "bfm_plan_run: null argument or bad batch size");
+    const int total = n_items * cfg->n_samples;
+    std::vector<bfm_plan_out> outs((size_t)total);
+    int rc = bfm_plan_layout(cfg, n_items, items, bufs, outs.data());
+    if (rc) return rc;
     int64_t used = arena_used_in, upload = 0;
     const int64_t start = (arena_used_in + 15) / 16 * 16;
-    int rc = bfm_plan_batch(cfg, n_items, items, outs.data(), seed, counter, arena_host, arena_dev, arena_capacity, &used,
-                            &upload, descs_host, descs_dev, info, nullptr, 0, nullptr);
+    rc = bfm_plan_batch(cfg, n_items, items, outs.data(), seed, counter, arena_host, arena_dev, arena_capacity, &used,
+                        &upload, descs_host, descs_dev, info, nullptr, 0, nullptr);
     if (rc) return rc;
     *arena_used_out = used;
     const int64_t nbytes = (upload + 15) / 16 * 16;

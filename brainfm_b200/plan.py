@@ -343,14 +343,6 @@ def set_zoom_tab(tab, tables, n_in, factors, n_out):
         tab.lo[ax], tab.hi[ax], tab.wl[ax], tab.wh[ax] = lo, hi, wl, wh
 
 
-def fill_zoom_tab(tab, arena, tables):
-    for ax, (lo, hi, wl, wh) in enumerate(tables):
-        tab.lo[ax] = arena.put(lo)
-        tab.hi[ax] = arena.put(hi)
-        tab.wl[ax] = arena.put(wl)
-        tab.wh[ax] = arena.put(wh)
-
-
 def make_deform(tables, arena, size, src, A, c2, fsmall_host, photo, F_full_ptr=None, fsmall_dev=None):
     """A filled _lib.Deform: the cached template of (size, small-grid shape) plus this sample's affine, source
     shape and small random grid (the only array that goes through the arena; fsmall_dev: it is already there)."""
@@ -366,51 +358,3 @@ def make_deform(tables, arena, size, src, A, c2, fsmall_host, photo, F_full_ptr=
     if fsmall_host is not None:
         d.fsmall = fsmall_dev if fsmall_dev is not None else arena.put(fsmall_host)
     return d
-
-
-def fill_deform(d, arena, size, src, A, c2, fsmall_host, photo, F_full_ptr=None, tables=None):
-    """Populate a _lib.Deform from host values (A, c2: float32 arrays as the reference's tensors).  With
-    `tables` (a DeviceTables) the zoom tables and candidate lists come from the device-resident cache and only
-    the small random grid goes through the arena."""
-    for a in range(3):
-        d.size[a] = int(size[a])
-        d.src[a] = int(src[a])
-        d.c2[a] = float(np.float32(c2[a]))
-        d.ctr[a] = float(np.float32((size[a] - 1) / 2))
-    Af = np.asarray(A, dtype=np.float32).reshape(-1)
-    for q in range(9):
-        d.A[q] = float(Af[q])
-    d.photo = int(bool(photo))
-    d.F_full = F_full_ptr
-    if F_full_ptr is not None:
-        for a in range(3):
-            d.ncand[a] = 0
-    elif fsmall_host is None:
-        for a in range(3):
-            if tables is not None:
-                d.cand[a], d.ncand[a] = tables.ends(size[a])
-            else:
-                d.cand[a] = arena.put(np.array([0, size[a] - 1], dtype=np.int32))
-                d.ncand[a] = 2
-    if fsmall_host is None:
-        d.fsmall = None
-        return
-    fs = fsmall_host.shape[:3]
-    for a in range(3):
-        d.fs[a] = int(fs[a])
-    d.fsmall = arena.put(fsmall_host.astype(np.float32, copy=False))
-    factor = np.array(size) / np.array(fs)
-    new = zoom_newsize(fs, factor)
-    assert tuple(new) == tuple(size), (new, size)
-    if tables is not None:
-        set_zoom_tab(d.ftab, tables, fs, factor, size)
-    else:
-        fill_zoom_tab(d.ftab, arena, [zoom_tables_host(fs[a], factor[a], int(new[a])) for a in range(3)])
-    if F_full_ptr is None:
-        for a in range(3):
-            if tables is not None:
-                d.cand[a], d.ncand[a] = tables.cand(fs[a], factor[a], int(new[a]))
-            else:
-                c = zoom_candidates_host(fs[a], factor[a], int(new[a]))
-                d.cand[a] = arena.put(c)
-                d.ncand[a] = int(c.size)

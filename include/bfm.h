@@ -429,8 +429,14 @@ typedef struct bfm_step_bufs {
     int64_t pair_ok;
 } bfm_step_bufs;
 
-/* bfm_plan_batch (native draws) + bfm_upload_pinned of the host-written arena prefix + bfm_gen_run, with the per-sample
- * buffers laid out from `bufs`: ONE call per batch.  items[n].aux_out / aux_raw are filled in.  arena_used_in: bytes of
+/* Lays the buffers of `bufs` out per sample: fills outs[0 .. n_items * cfg->n_samples) and items[n].aux_out / aux_raw
+ * of every fused real-image target, in item order (what bfm_plan_batch takes).  Refuses a null out / syn / i_bf / tmp /
+ * lowres, and a null aux_out / aux_raw when an item has such a target. */
+int bfm_plan_layout(const bfm_plan_cfg *cfg, int n_items, bfm_plan_item *items, const bfm_step_bufs *bufs,
+                    bfm_plan_out *outs);
+
+/* bfm_plan_layout + bfm_plan_batch (native draws) + bfm_upload_pinned of the host-written arena prefix + bfm_gen_run:
+ * ONE call per batch.  items[n].aux_out / aux_raw are filled in.  arena_used_in: bytes of
  * the arena already reserved; *arena_used_out: after planning. */
 int bfm_plan_run(const bfm_plan_cfg *cfg, int n_items, bfm_plan_item *items, const bfm_step_bufs *bufs, uint64_t seed,
                  uint64_t counter, void *arena_host, void *arena_dev, int64_t arena_capacity, int64_t arena_used_in,

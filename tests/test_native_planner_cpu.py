@@ -267,3 +267,68 @@ def test_misaligned_buffers_are_refused_before_any_launch(field):
                   L.bfm_gen_finish):
         assert stage(C.addressof(r['descs']), FAKE, 1, None) == _lib.BFM_E_INVALID
         assert "misaligned" in L.bfm_last_error().decode()
+
+
+def test_layout_of_the_per_sample_buffers():
+    """bfm_plan_layout, the one per-sample buffer layout of both batch paths (bfm_plan_run, NativePlanner.run): outputs
+    advance by N floats per sample, the scratch by Npad = N rounded up to a multiple of 4 (two slots per sample for
+    tmp), syn by syn_stride, and the fused targets by N / Npad per target in item order.  N is odd here (91 x 109 x 91)
+    so that N and Npad differ."""
+    L = _lib.lib()
+    cfg = _lib.PlanCfg()
+    cfg.size[:] = [91, 109, 91]
+    cfg.n_samples = 2
+    N = 91 * 109 * 91
+    Np = N + 3
+    assert N % 2 == 1 and Np % 4 == 0
+    n_aux = [2, 0, 3]
+    items = (_lib.PlanItem * 3)()
+    for it, k in zip(items, n_aux):
+        it.n_aux = k
+    names = ("out", "bflog_out", "residual", "syn", "i_bf", "tmp", "lowres", "aux_out", "aux_raw")
+    base = {f: FAKE + (k << 36) for k, f in enumerate(names)}
+    stride = 2 * 902912                          # syn: float2 pairs of a padded source volume
+
+    def layout(n_items=3, **over):
+        bufs = _lib.StepBufs(**dict(base, **over))
+        bufs.syn_stride, bufs.pair_ok = stride, 1
+        outs = (_lib.PlanOut * (max(n_items, 1) * 2))()
+        return L.bfm_plan_layout(C.addressof(cfg), n_items, C.addressof(items), C.addressof(bufs),
+                                 C.addressof(outs)), outs
+
+    rc, outs = layout()
+    assert rc == _lib.BFM_OK
+    for q in range(6):
+        o = outs[q]
+        assert (o.out, o.bflog_out, o.residual) == tuple(base[f] + 4 * q * N for f in ("out", "bflog_out", "residual"))
+        assert o.syn == base["syn"] + 4 * q * stride and o.syn_pair_ok == 1
+        assert o.i_bf == base["i_bf"] + 4 * q * Np and o.lowres == base["lowres"] + 4 * q * Np
+        assert o.tmp[0] == base["tmp"] + 4 * (2 * q) * Np and o.tmp[1] == base["tmp"] + 4 * (2 * q + 1) * Np
+    k = 0
+    for it in items:
+        for c in range(_lib.MAX_AUX):
+            if c < it.n_aux:
+                assert it.aux_out[c] == base["aux_out"] + 4 * k * N and it.aux_raw[c] == base["aux_raw"] + 4 * k * Np
+                k += 1
+            else:
+                assert it.aux_out[c] is None and it.aux_raw[c] is None
+    assert k == 5
+    # no bias-field log / residual output requested: null in every sample
+    rc, outs = layout(bflog_out=None, residual=None)
+    assert rc == _lib.BFM_OK and all(o.bflog_out is None and o.residual is None for o in outs)
+    # refusals
+    for f in ("out", "syn", "i_bf", "tmp", "lowres"):
+        assert layout(**{f: None})[0] == _lib.BFM_E_INVALID and "null buffer" in L.bfm_last_error().decode()
+    for f in ("aux_out", "aux_raw"):
+        assert layout(**{f: None})[0] == _lib.BFM_E_INVALID and "null target" in L.bfm_last_error().decode()
+        assert layout(n_items=2, **{f: None})[0] == _lib.BFM_E_INVALID      # item 0 has targets
+    items[0].n_aux = 0
+    assert layout(n_items=2, aux_out=None, aux_raw=None)[0] == _lib.BFM_OK      # no target in the batch
+    for n_items in (0, -1, 4097):
+        assert layout(n_items=n_items)[0] == _lib.BFM_E_INVALID
+    bufs, outs = _lib.StepBufs(**base), (_lib.PlanOut * 6)()
+    for args in ((None, 3, C.addressof(items), C.addressof(bufs), C.addressof(outs)),
+                 (C.addressof(cfg), 3, None, C.addressof(bufs), C.addressof(outs)),
+                 (C.addressof(cfg), 3, C.addressof(items), None, C.addressof(outs)),
+                 (C.addressof(cfg), 3, C.addressof(items), C.addressof(bufs), None)):
+        assert L.bfm_plan_layout(*args) == _lib.BFM_E_INVALID
